@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K --warmup W   # the reference's CPU path (port)
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   # also write the last timed step's results (dump_outputs)
 
 A "step" is one training step (forward, CrossEntropy, backward, Adam) of MedMamba-T
 (MedMamba.py VSSM, depths 2-2-4-2, dims 96-768, 6 classes) on synthetic 3x224x224 images,
@@ -346,6 +347,49 @@ def run_reference(args):
 
 
 # ------------------------------------------------------------------------------------------------
+# --dump-outputs: what the last timed step computed, for comparing two builds output for output
+# ------------------------------------------------------------------------------------------------
+DUMP_SAMPLE = 1 << 23      # elements kept of the flattened gradients: 32 MiB of float32
+
+
+def restore_initial_state(net, opt, init_state):
+    """Puts the model back to its seeded initial parameters and buffers and the optimizer back to a fresh state, in place (the
+    captured step graph keeps reading the same tensors).  The step that --dump-outputs records starts from here, so its inputs are
+    the same in every run: the backward kernels sum dB / dC / dA and the weight gradients with float atomics, in no fixed order,
+    and Adam on the benchmark's one repeated batch turns those last-bit differences into large ones within a few steps."""
+    import torch
+    with torch.no_grad():
+        for k, v in net.state_dict().items():
+            v.copy_(init_state[k])
+        for st in opt.state.values():           # Adam: step, exp_avg, exp_avg_sq
+            for t in st.values():
+                if torch.is_tensor(t):
+                    t.zero_()
+
+
+def dump_outputs(out_dir, loss, net):
+    """Writes, as float32 .npy files, what the last timed step computed from the seeded model and batch:
+      loss.npy     the loss the step returned, shape (1,)
+      grads.npy    the parameters' gradients (zeros for a parameter that received none), flattened in named_parameters() order
+      buffers.npy  the floating-point buffers (BatchNorm running statistics its forward updated), flattened in named_buffers() order
+    Gradients larger than DUMP_SAMPLE elements keep the same DUMP_SAMPLE positions, drawn once from a fixed seed, so two runs of
+    the same model are compared element for element."""
+    import numpy as np
+    import torch
+    params = [p for _, p in net.named_parameters()]
+    flat_g = torch.cat([(p.grad if p.grad is not None else torch.zeros_like(p)).detach().float().reshape(-1) for p in params])
+    if flat_g.numel() > DUMP_SAMPLE:
+        keep = np.sort(np.random.default_rng(0).choice(flat_g.numel(), DUMP_SAMPLE, replace=False))
+        flat_g = flat_g[torch.from_numpy(keep).to(flat_g.device)]
+    bufs = [b.detach().float().reshape(-1) for _, b in net.named_buffers() if b.is_floating_point()]
+    arrays = {"loss": loss.detach().float().reshape(1), "grads": flat_g,
+              "buffers": torch.cat(bufs) if bufs else torch.zeros(0, device=flat_g.device)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy().astype(np.float32))
+
+
+# ------------------------------------------------------------------------------------------------
 # this repo's arm
 # ------------------------------------------------------------------------------------------------
 def run_cuda(args):
@@ -393,6 +437,7 @@ def run_cuda(args):
                      bucket_cap_mb=args.bucket_mb, grad_bf16=args.grad_bf16, broadcast_buffers=args.broadcast_buffers,
                      ddp_impl=args.ddp_impl)
     model = step.model
+    init_state = {k: v.detach().clone() for k, v in net.state_dict().items()} if args.dump_outputs else None
     B = args.batch
     x_dev = torch.randn(B, 3, 224, 224, device=dev)
     y_dev = torch.randint(0, NUM_CLASSES, (B,), device=dev)
@@ -420,12 +465,23 @@ def run_cuda(args):
     barrier()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    for _ in range(args.steps):
+    for _ in range(args.steps - (init_state is not None)):
         run_step(xin, yin)
     e1.record()
+    if init_state is not None:
+        # the last timed step, timed on its own: it starts from the seeded initial state (restored outside the timing)
+        restore_initial_state(net, step.opt, init_state)
+        d0, d1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        d0.record()
+        loss = run_step(xin, yin)
+        d1.record()
     barrier()
     launches = _lib.launches() - launches0
     ms = e0.elapsed_time(e1)
+    if init_state is not None:
+        ms += d0.elapsed_time(d1)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, loss, net)   # before region 2 trains the model further
     # ---- timed region 2: end to end (pinned host input -> device, loss -> host) ----
     barrier()
     f0, f1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -548,7 +604,14 @@ def main():
     ap.add_argument("--grad-bf16", action="store_true", help="bf16-compressed gradient all-reduce (N > 1)")
     ap.add_argument("--broadcast-buffers", action="store_true",
                     help="re-enable DDP's per-step broadcast of rank 0's BatchNorm statistics (N > 1; see train_step.py)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss, gradients and BatchNorm buffers of the last timed step as DIR/<name>.npy (float32); that step "
+                         "starts from the seeded initial model and a fresh optimizer, so runs with the same arguments compare")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the CUDA training step computed: it does not apply to --impl reference")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -121,8 +121,10 @@ def test_bf16_autocast_model_matches_reference():
 
 def test_backward_inside_autocast_region_is_safe():
     """ADVICE r1: loss.backward() called INSIDE the autocast block runs the custom backwards under autocast; the ctypes-backed
-    Functions must not hand re-cast (bf16) buffers to fp32 kernels.  Gradients must equal the backward-outside run bit for bit
-    up to atomics order."""
+    Functions must not hand re-cast (bf16) buffers to fp32 kernels.  Gradients must equal the backward-outside run up to the order
+    of the fp32 atomics, and meet the bf16 bars against the fp32 reference golden.  The two runs are compared by direction
+    (cosine) rather than element by element: under bf16 autocast a last-bit difference from the atomics can flip one bf16
+    rounding downstream and move single elements by ~2^-8 of their magnitude, while a mis-cast buffer scrambles whole tensors."""
     net, x, y, g = _setup()
     net.train()
     with torch.autocast("cuda", dtype=torch.bfloat16):
@@ -133,11 +135,23 @@ def test_backward_inside_autocast_region_is_safe():
     with torch.autocast("cuda", dtype=torch.bfloat16):
         loss2 = torch.nn.functional.cross_entropy(net(x).float(), y)
         loss2.backward()
-    gmax = max(float(v.float().abs().max()) for v in ref.values())
+    assert set(ref) == {k for k, p in net.named_parameters() if p.grad is not None}
+    nmax = max(float(v.float().norm()) for v in ref.values())
+    cos, allg, allr = {}, [], []
     for k, p in net.named_parameters():
         if p.grad is None:
             continue
         assert torch.isfinite(p.grad).all(), k
-        a, b = p.grad.float(), ref[k].float()
-        # same kernels, same inputs: only the order of the fp32 atomics differs between the two runs
-        assert float((a - b).abs().max()) <= 2e-3 * float(b.abs().max()) + 1e-6 * gmax, k
+        a, b = p.grad.float().cpu().numpy(), ref[k].float().cpu().numpy()
+        allg.append(a.ravel()); allr.append(b.ravel())
+        if float(ref[k].float().norm()) > 1e-3 * nmax:
+            cos[k] = _cos(a, b)
+    worst = min(cos, key=cos.get)
+    cos_all = _cos(np.concatenate(allg), np.concatenate(allr))
+    gcos, gcos_all, n = _grad_report(net, g)
+    gworst = min(gcos, key=gcos.get)
+    print(f"backward inside vs outside autocast: global grad cosine {cos_all:.7f}, worst per-parameter cosine {cos[worst]:.7f} ({worst}) "
+          f"over {len(cos)} parameters; vs the fp32 golden: global {gcos_all:.5f}, worst {gcos[gworst]:.5f} ({gworst})")
+    # same kernels, same inputs: only the order of the fp32 atomics differs between the two runs
+    assert cos_all > 0.99999 and cos[worst] > 0.999, (cos_all, worst, cos[worst])
+    assert n > 60 and gcos_all > 0.99 and gcos[gworst] > 0.95, (gcos_all, gworst, gcos[gworst])

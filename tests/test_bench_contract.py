@@ -36,6 +36,54 @@ def test_product_arm_needs_a_gpu():
     assert not [l for l in out.stdout.splitlines() if l.startswith("{") and '"value"' in l]
 
 
+def test_dump_outputs_writer_and_state_restore(tmp_path, monkeypatch):
+    """CPU: bench.dump_outputs writes float32 loss / grads / buffers, sampling the gradients at the same seeded positions on every
+    call; bench.restore_initial_state brings back the seeded weights and buffers and a fresh Adam state in place."""
+    import numpy as np
+    import torch
+    import bench
+    from medical_image_classification_b200.models import VSSM
+    torch.manual_seed(0)
+    net = VSSM(num_classes=6, depths=[1, 1], dims=[16, 32], drop_path_rate=0.0)
+    init = {k: v.detach().clone() for k, v in net.state_dict().items()}
+    ptrs = [p.data_ptr() for p in net.parameters()]
+    opt = torch.optim.Adam(net.parameters(), lr=1e-2)
+    for _ in range(2):
+        for p in net.parameters():
+            p.grad = torch.randn_like(p)
+        opt.step()
+    net.state_dict()[next(k for k in init if k.endswith("running_mean"))].add_(1.0)
+    bench.restore_initial_state(net, opt, init)
+    assert [p.data_ptr() for p in net.parameters()] == ptrs
+    assert all(torch.equal(v, init[k]) for k, v in net.state_dict().items())
+    assert all(not t.any() for st in opt.state.values() for t in st.values() if torch.is_tensor(t))
+
+    params = list(net.parameters())
+    params[0].grad = None                                        # a parameter without a gradient is dumped as zeros
+    flat = torch.cat([(p.grad if p.grad is not None else torch.zeros_like(p)).reshape(-1) for p in params]).numpy()
+    monkeypatch.setattr(bench, "DUMP_SAMPLE", 1000)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), torch.tensor(1.25), net)
+    a = {n: np.load(tmp_path / "a" / f"{n}.npy") for n in ("loss", "grads", "buffers")}
+    assert sorted(os.listdir(tmp_path / "a")) == ["buffers.npy", "grads.npy", "loss.npy"]
+    assert all(v.dtype == np.float32 for v in a.values())
+    assert a["loss"].tolist() == [1.25] and a["grads"].shape == (1000,)
+    assert a["buffers"].size == sum(b.numel() for b in net.buffers() if b.is_floating_point())
+    for n, v in a.items():
+        assert np.array_equal(v, np.load(tmp_path / "b" / f"{n}.npy")), n
+    keep = np.sort(np.random.default_rng(0).choice(flat.size, 1000, replace=False))
+    assert np.array_equal(a["grads"], flat[keep])
+    monkeypatch.setattr(bench, "DUMP_SAMPLE", flat.size)         # at or under the limit: every element, in order
+    bench.dump_outputs(str(tmp_path / "c"), torch.tensor(1.25), net)
+    assert np.array_equal(np.load(tmp_path / "c" / "grads.npy"), flat)
+
+
+def test_bench_rejects_meaningless_arguments():
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "unused"]):
+        out = subprocess.run([sys.executable, "bench.py", *extra], cwd=ROOT, capture_output=True, text=True, timeout=120)
+        assert out.returncode == 2 and "error" in out.stderr, extra
+
+
 def test_reference_arm_medssd():
     """BASELINE.json configs[2]: the same arm for the SSD family (eager CPU tree + the from-definition SSD oracle)."""
     out = subprocess.run([sys.executable, "bench.py", "--impl", "reference", "--model", "medssd", "--steps", "1", "--warmup", "0",
