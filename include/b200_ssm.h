@@ -124,9 +124,12 @@ size_t b200_sscan_ckpt_bytes(int32_t batch, int32_t dim, int32_t seqlen, int32_t
                              int32_t n_groups, int32_t ckpt_every);
 int b200_sscan_fwd(const b200_sscan_fwd_params* p, b200_stream_t stream);
 int b200_sscan_bwd(const b200_sscan_bwd_params* p, b200_stream_t stream);
-/* Which kernel generation the calling thread's last b200_sscan_fwd / _bwd launched: 2 = the TMA-staged kernels of sscan2.cu
- * (fp32 tensors whose layouts tensor maps can describe: L % 4 == 0, 16-byte aligned bases and strides), 1 = sscan.cu (every other
- * layout, 16-bit I/O, the z gate in the backward).  Both generations share the checkpoint format; for profilers and tests. */
+/* Which kernel the calling thread's last b200_sscan_fwd / _bwd launched:
+ *   1 = sscan.cu (every layout sscan2.cu cannot take: L % 4 != 0, unaligned views, 16-bit I/O, the z gate in the backward),
+ *   2 = the TMA-staged kernels of sscan2.cu (fp32 tensors whose layouts tensor maps can describe: L % 4 == 0, 16-byte aligned
+ *       bases and strides),
+ *   3 = sscan.cu with its opt-in TMA row staging (B200_SSCAN_TMA=1, fp32 with tensor-map-describable u / delta / dout).
+ * Both generations share the checkpoint format; for profilers and tests. */
 int b200_sscan_last_variant(void);
 
 /* ------------------------------------------------------------------------------------------

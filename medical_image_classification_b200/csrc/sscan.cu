@@ -1035,6 +1035,9 @@ static bool make_fwd_maps(RowMaps* tm, const b200_sscan_fwd_params* p) {
                         p->delta_group_stride, p->delta_batch_stride);
 }
 
+// b200_sscan_last_variant(): 1 = sscan.cu, 2 = sscan2.cu, 3 = sscan.cu with the TMA row staging (include/b200_ssm.h)
+static thread_local int g_last_variant = 0;
+
 template <typename T>
 static int launch_fwd(const b200_sscan_fwd_params* p, cudaStream_t st) {
     const long long nt = n_tasks(p);
@@ -1042,6 +1045,7 @@ static int launch_fwd(const b200_sscan_fwd_params* p, cudaStream_t st) {
     RowMaps tm;
     memset(&tm, 0, sizeof(tm));
     const bool use_tma = sizeof(T) == 4 && make_fwd_maps(&tm, p);
+    g_last_variant = use_tma ? 3 : 1;
     if (use_tma) {
         if (p->z) sscan_fwd_kernel<T, true, sizeof(T) == 4><<<grid, WPB * 32, 0, st>>>(*p, tm);
         else sscan_fwd_kernel<T, false, sizeof(T) == 4><<<grid, WPB * 32, 0, st>>>(*p, tm);
@@ -1068,6 +1072,7 @@ static int launch_bwd(const b200_sscan_bwd_params* q, cudaStream_t st) {
                                       q->dout_row_stride, q->dout_group_stride, q->dout_batch_stride))
                             ? 1
                             : 0;
+    g_last_variant = use_tma && sizeof(T) == 4 ? 3 : 1;
     if (use_tma && sizeof(T) == 4) {
         if (q->f.z) sscan_bwd_kernel<T, true, sizeof(T) == 4><<<grid, WPB * 32, 0, st>>>(*q, tm);
         else sscan_bwd_kernel<T, false, sizeof(T) == 4><<<grid, WPB * 32, 0, st>>>(*q, tm);
@@ -1089,7 +1094,6 @@ bool try_bwd(const b200_sscan_bwd_params* q, cudaStream_t st, int* rc);
 
 using namespace b200;
 
-static thread_local int g_last_variant = 0;
 extern "C" int b200_sscan_last_variant(void) { return g_last_variant; }
 
 extern "C" size_t b200_sscan_ckpt_bytes(int32_t batch, int32_t dim, int32_t seqlen, int32_t dstate, int32_t n_groups,
@@ -1115,7 +1119,6 @@ extern "C" int b200_sscan_fwd(const b200_sscan_fwd_params* p, b200_stream_t stre
             return rc;
         }
     }
-    g_last_variant = 1;
     switch (p->io_dtype) {
         case B200_F32: return launch_fwd<float>(p, st);
         case B200_BF16: return launch_fwd<__nv_bfloat16>(p, st);
@@ -1143,7 +1146,6 @@ extern "C" int b200_sscan_bwd(const b200_sscan_bwd_params* q, b200_stream_t stre
             return rc;
         }
     }
-    g_last_variant = 1;
     switch (q->f.io_dtype) {
         case B200_F32: return launch_bwd<float>(q, st);
         case B200_BF16: return launch_bwd<__nv_bfloat16>(q, st);
