@@ -74,19 +74,45 @@ class SsdBwdParams(C.Structure):
 
 _DTYPES = {torch.float32: 0, torch.bfloat16: 1, torch.float16: 2}
 
-# every symbol include/b200_ssm.h declares
-EXPORTS = [
-    "b200_sscan_ckpt_bytes", "b200_sscan_fwd", "b200_sscan_bwd", "b200_sscan_last_variant",
-    "b200_cross_scan_pack", "b200_cross_scan_pack_bwd", "b200_cross_merge", "b200_cross_merge_bwd",
-    "b200_cross_scan4", "b200_cross_scan4_bwd", "b200_ssd_merge4", "b200_ssd_merge4_bwd",
-    "b200_ssd_workspace_bytes", "b200_ssd_bwd_scratch_bytes", "b200_ssd_fwd", "b200_ssd_bwd",
-    "b200_rmsnorm_gated_fwd", "b200_rmsnorm_gated_bwd",
-    "b200_cross_scan_pack_strided", "b200_cross_scan_unpack4", "b200_atrous_scan", "b200_atrous_merge",
-    "b200_ln_gate_grid", "b200_ln_gate_fwd", "b200_ln_gate_bwd",
-    "b200_dwconv_silu_fwd", "b200_dwconv_silu_bwd",
-    "b200_shuffle_cat_add_fwd", "b200_shuffle_cat_add_bwd", "b200_patch_merge",
-    "b200_last_error", "b200_version", "b200_kernel_launches", "b200_sizeof_params",
-]
+# name -> (restype, argtypes) of every function include/b200_ssm.h declares, in the header's order
+# (tests/test_abi.py parses the header and checks each entry)
+SIGNATURES = {
+    "b200_sscan_ckpt_bytes": (C.c_size_t, [i32] * 6),
+    "b200_sscan_fwd": (C.c_int, [C.POINTER(SScanFwdParams), vp]),
+    "b200_sscan_bwd": (C.c_int, [C.POINTER(SScanBwdParams), vp]),
+    "b200_sscan_last_variant": (C.c_int, []),
+    "b200_cross_scan_pack_strided": (C.c_int, [vp, vp, i64, i64, i64, i32, i32, i32, i32, vp]),
+    "b200_cross_scan_unpack4": (C.c_int, [vp, vp, i64, i64, i64, vp, i32, i32, i32, i32, vp]),
+    "b200_atrous_scan": (C.c_int, [vp, vp, i32, i32, i32, i32, i32, vp]),
+    "b200_atrous_merge": (C.c_int, [vp, vp, i32, i32, i32, i32, i32, vp]),
+    "b200_cross_scan_pack": (C.c_int, [vp, vp, i32, i32, i32, i32, i32, vp]),
+    "b200_cross_scan_pack_bwd": (C.c_int, [vp, vp, i32, i32, i32, i32, i32, vp]),
+    "b200_cross_merge": (C.c_int, [vp, vp, i32, i32, i32, i32, i32, vp]),
+    "b200_cross_merge_bwd": (C.c_int, [vp, vp, i32, i32, i32, i32, i32, vp]),
+    "b200_cross_scan4": (C.c_int, [vp, i64, vp, i32, i32, i32, i32, vp]),
+    "b200_cross_scan4_bwd": (C.c_int, [vp, vp, i64, i32, i32, i32, i32, vp]),
+    "b200_ssd_merge4": (C.c_int, [vp, vp, i32, i32, i32, i32, vp]),
+    "b200_ssd_merge4_bwd": (C.c_int, [vp, vp, i32, i32, i32, i32, vp]),
+    "b200_ssd_workspace_bytes": (C.c_size_t, [i32] * 7),
+    "b200_ssd_bwd_scratch_bytes": (C.c_size_t, [i32] * 7),
+    "b200_ssd_fwd": (C.c_int, [C.POINTER(SsdFwdParams), vp]),
+    "b200_ssd_bwd": (C.c_int, [C.POINTER(SsdBwdParams), vp]),
+    "b200_rmsnorm_gated_fwd": (C.c_int, [vp, vp, vp, vp, vp, i64, i32, f32, vp]),
+    "b200_rmsnorm_gated_bwd": (C.c_int, [vp, vp, vp, vp, vp, vp, vp, vp, i32, i64, i32, vp]),
+    "b200_ln_gate_grid": (C.c_int, [i64]),
+    "b200_ln_gate_fwd": (C.c_int, [vp, i32, i64, vp, i64, i32, vp, vp, vp, i32, vp, vp, i64, i32, f32, vp]),
+    "b200_ln_gate_bwd": (C.c_int, [vp, vp, i32, i64, vp, i64, i32, vp, vp, i32, vp, vp, vp, vp, vp, vp, i64, i32, vp]),
+    "b200_dwconv_silu_fwd": (C.c_int, [vp, i64, i32, vp, vp, vp, i32, i32, i32, i32, vp]),
+    "b200_dwconv_silu_bwd": (C.c_int, [vp, vp, i64, i32, vp, vp, vp, vp, vp, i32, i32, i32, i32, vp]),
+    "b200_shuffle_cat_add_fwd": (C.c_int, [vp, i32, vp, i32, vp, vp, i32, i32, i32, i32, vp]),
+    "b200_shuffle_cat_add_bwd": (C.c_int, [vp, i32, vp, i32, vp, i32, i32, i32, i32, vp]),
+    "b200_patch_merge": (C.c_int, [vp, vp, i32, i32, i32, i32, i32, vp]),
+    "b200_last_error": (C.c_char_p, []),
+    "b200_version": (C.c_int, []),
+    "b200_kernel_launches": (C.c_int, []),
+    "b200_sizeof_params": (C.c_size_t, [i32]),
+}
+EXPORTS = list(SIGNATURES)
 
 _lib = None
 
@@ -109,39 +135,9 @@ def load() -> C.CDLL:
     elif not os.path.exists(LIB_PATH):
         raise RuntimeError(f"{LIB_PATH} is missing and nvcc is not available to build it: there is no fallback path")
     lib = C.CDLL(LIB_PATH)
-    lib.b200_last_error.restype = C.c_char_p
-    lib.b200_sscan_ckpt_bytes.restype = C.c_size_t
-    lib.b200_sscan_ckpt_bytes.argtypes = [i32] * 6
-    lib.b200_ssd_workspace_bytes.restype = C.c_size_t
-    lib.b200_ssd_workspace_bytes.argtypes = [i32] * 7
-    lib.b200_ssd_bwd_scratch_bytes.restype = C.c_size_t
-    lib.b200_ssd_bwd_scratch_bytes.argtypes = [i32] * 7
-    lib.b200_sizeof_params.restype = C.c_size_t
-    lib.b200_sizeof_params.argtypes = [i32]
-    lib.b200_sscan_fwd.argtypes = [C.POINTER(SScanFwdParams), vp]
-    lib.b200_sscan_bwd.argtypes = [C.POINTER(SScanBwdParams), vp]
-    lib.b200_ssd_fwd.argtypes = [C.POINTER(SsdFwdParams), vp]
-    lib.b200_ssd_bwd.argtypes = [C.POINTER(SsdBwdParams), vp]
-    for name in ("b200_cross_scan_pack", "b200_cross_scan_pack_bwd", "b200_cross_merge", "b200_cross_merge_bwd"):
-        getattr(lib, name).argtypes = [vp, vp, i32, i32, i32, i32, i32, vp]
-    lib.b200_cross_scan4.argtypes = [vp, i64, vp, i32, i32, i32, i32, vp]
-    lib.b200_cross_scan4_bwd.argtypes = [vp, vp, i64, i32, i32, i32, i32, vp]
-    lib.b200_ssd_merge4.argtypes = [vp, vp, i32, i32, i32, i32, vp]
-    lib.b200_ssd_merge4_bwd.argtypes = [vp, vp, i32, i32, i32, i32, vp]
-    lib.b200_rmsnorm_gated_fwd.argtypes = [vp, vp, vp, vp, vp, i64, i32, f32, vp]
-    lib.b200_rmsnorm_gated_bwd.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, i32, i64, i32, vp]
-    lib.b200_dwconv_silu_fwd.argtypes = [vp, i64, i32, vp, vp, vp, i32, i32, i32, i32, vp]
-    lib.b200_dwconv_silu_bwd.argtypes = [vp, vp, i64, i32, vp, vp, vp, vp, vp, i32, i32, i32, i32, vp]
-    lib.b200_shuffle_cat_add_fwd.argtypes = [vp, i32, vp, i32, vp, vp, i32, i32, i32, i32, vp]
-    lib.b200_shuffle_cat_add_bwd.argtypes = [vp, i32, vp, i32, vp, i32, i32, i32, i32, vp]
-    lib.b200_patch_merge.argtypes = [vp, vp, i32, i32, i32, i32, i32, vp]
-    lib.b200_atrous_scan.argtypes = [vp, vp, i32, i32, i32, i32, i32, vp]
-    lib.b200_atrous_merge.argtypes = [vp, vp, i32, i32, i32, i32, i32, vp]
-    lib.b200_cross_scan_pack_strided.argtypes = [vp, vp, i64, i64, i64, i32, i32, i32, i32, vp]
-    lib.b200_cross_scan_unpack4.argtypes = [vp, vp, i64, i64, i64, vp, i32, i32, i32, i32, vp]
-    lib.b200_ln_gate_grid.argtypes = [i64]
-    lib.b200_ln_gate_fwd.argtypes = [vp, i32, i64, vp, i64, i32, vp, vp, vp, i32, vp, vp, i64, i32, f32, vp]
-    lib.b200_ln_gate_bwd.argtypes = [vp, vp, i32, i64, vp, i64, i32, vp, vp, i32, vp, vp, vp, vp, vp, vp, i64, i32, vp]
+    for name, (restype, argtypes) in SIGNATURES.items():
+        fn = getattr(lib, name)
+        fn.restype, fn.argtypes = restype, argtypes
     for which, st in enumerate((SScanFwdParams, SScanBwdParams, SsdFwdParams, SsdBwdParams)):
         if lib.b200_sizeof_params(which) != C.sizeof(st):
             raise RuntimeError(f"libb200ssm ABI mismatch for {st.__name__}: "
@@ -156,6 +152,14 @@ def check(rc: int, what: str) -> None:
         raise RuntimeError(f"{what} failed (rc={rc}): {msg}")
 
 
+def launch(name: str, device, *args) -> None:
+    """Call the entry point `name` with `args` and the current stream of `device`, with `device` current; raise on an error."""
+    lib = load()
+    with torch.cuda.device(device):
+        rc = getattr(lib, name)(*args, stream_ptr(device))
+    check(rc, name)
+
+
 def ptr(t):
     return None if t is None else t.data_ptr()
 
@@ -168,6 +172,21 @@ def require_cuda(*tensors) -> None:
     for t in tensors:
         if t is not None and not t.is_cuda:
             raise RuntimeError("libb200ssm ops run on CUDA tensors only: there is no CPU fallback")
+
+
+def f32c(t):
+    """t as a detached contiguous fp32 tensor (the layout the kernels read A, D and biases in); None stays None."""
+    return None if t is None else t.detach().to(torch.float32).contiguous()
+
+
+def is_dense(t) -> bool:
+    """True when the tensor's elements fill one contiguous block exactly once (any dimension order, e.g. channels_last)."""
+    expect = 1
+    for size, stride in sorted(((sz, st) for sz, st in zip(t.shape, t.stride()) if sz != 1), key=lambda e: e[1]):
+        if stride != expect:
+            return False
+        expect *= size
+    return True
 
 
 def no_autocast(fn):

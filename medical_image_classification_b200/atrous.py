@@ -20,12 +20,6 @@ from . import _lib
 from .selective_scan_interface import selective_scan_fn
 
 
-def _op(name, src, dst, B, C, H, W):
-    lib = _lib.load()
-    with torch.cuda.device(src.device):
-        _lib.check(getattr(lib, name)(src.data_ptr(), dst.data_ptr(), B, C, H, W, _lib.dtype_code(src.dtype), _lib.stream_ptr(src.device)), name)
-
-
 def _check_step(step_size):
     if step_size != 2:
         raise RuntimeError(f"atrous scan: step_size {step_size} is not supported by the B200 kernels (the reference uses 2)")
@@ -43,7 +37,7 @@ class EfficientScan(torch.autograd.Function):
         B, C, H, W = x.shape
         L2 = math.ceil(H / 2) * math.ceil(W / 2)
         xs = torch.empty((B, 4, C, L2), dtype=x.dtype, device=x.device)
-        _op("b200_atrous_scan", x, xs, B, C, H, W)
+        _lib.launch("b200_atrous_scan", x.device, x.data_ptr(), xs.data_ptr(), B, C, H, W, _lib.dtype_code(x.dtype))
         ctx.shape = (B, C, H, W)
         return xs
 
@@ -53,7 +47,7 @@ class EfficientScan(torch.autograd.Function):
         B, C, H, W = ctx.shape
         grad_xs = grad_xs.contiguous()
         gx = torch.empty((B, C, H, W), dtype=grad_xs.dtype, device=grad_xs.device)
-        _op("b200_atrous_merge", grad_xs, gx, B, C, H, W)
+        _lib.launch("b200_atrous_merge", grad_xs.device, grad_xs.data_ptr(), gx.data_ptr(), B, C, H, W, _lib.dtype_code(grad_xs.dtype))
         return gx, None
 
 
@@ -71,7 +65,7 @@ class EfficientMerge(torch.autograd.Function):
         if K != 4 or L2 != math.ceil(H / 2) * math.ceil(W / 2):
             raise RuntimeError(f"EfficientMerge: ys {tuple(ys.shape)} does not match a {H} x {W} image")
         y = torch.empty((B, C, H, W), dtype=ys.dtype, device=ys.device)
-        _op("b200_atrous_merge", ys, y, B, C, H, W)
+        _lib.launch("b200_atrous_merge", ys.device, ys.data_ptr(), y.data_ptr(), B, C, H, W, _lib.dtype_code(ys.dtype))
         ctx.shape = (B, C, H, W)
         return y.view(B, C, H * W)
 
@@ -82,7 +76,7 @@ class EfficientMerge(torch.autograd.Function):
         grad_y = grad_y.contiguous()
         L2 = math.ceil(H / 2) * math.ceil(W / 2)
         gys = torch.empty((B, 4, C, L2), dtype=grad_y.dtype, device=grad_y.device)
-        _op("b200_atrous_scan", grad_y, gys, B, C, H, W)
+        _lib.launch("b200_atrous_scan", grad_y.device, grad_y.data_ptr(), gys.data_ptr(), B, C, H, W, _lib.dtype_code(grad_y.dtype))
         return gys, None, None, None
 
 

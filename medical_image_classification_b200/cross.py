@@ -1,4 +1,4 @@
-"""SS2D cross-scan / selective scan / cross-merge as two autograd Functions over libb200ssm.
+"""SS2D cross-scan / selective scan / cross-merge as autograd Functions over libb200ssm.
 
 Reference semantics (MedMamba.py:386-424, 476-477): four orderings of every channel plane --
 k=0 row-major, k=1 column-major, k=2/3 their time reversals -- are scanned independently and the
@@ -18,18 +18,10 @@ import torch
 
 from ._lib import no_autocast as _no_autocast
 from . import _lib
-from .selective_scan_interface import _f32c, launch_bwd, launch_fwd
+from .selective_scan_interface import launch_bwd, launch_fwd
 
 DIR_PERM = (0, 2, 1, 3)   # internal direction -> reference direction k (self-inverse)
 REV_MASK = 0b1010         # internal directions 1 and 3 run backwards in time
-
-
-def _plane_op(name, src, dst, batch, D, H, W):
-    lib = _lib.load()
-    with torch.cuda.device(src.device):
-        rc = getattr(lib, name)(src.data_ptr(), dst.data_ptr(), batch, D, H, W, _lib.dtype_code(src.dtype),
-                                _lib.stream_ptr(src.device))
-    _lib.check(rc, name)
 
 
 class CrossScanPackFn(torch.autograd.Function):
@@ -42,7 +34,7 @@ class CrossScanPackFn(torch.autograd.Function):
         x = x.contiguous()
         B, D, H, W = x.shape
         x2 = torch.empty((B, 2, D, H * W), dtype=x.dtype, device=x.device)
-        _plane_op("b200_cross_scan_pack", x, x2, B, D, H, W)
+        _lib.launch("b200_cross_scan_pack", x.device, x.data_ptr(), x2.data_ptr(), B, D, H, W, _lib.dtype_code(x.dtype))
         ctx.hw = (H, W)
         return x2
 
@@ -53,7 +45,7 @@ class CrossScanPackFn(torch.autograd.Function):
         dx2 = dx2.contiguous()
         B, _, D, _ = dx2.shape
         dx = torch.empty((B, D, H, W), dtype=dx2.dtype, device=dx2.device)
-        _plane_op("b200_cross_scan_pack_bwd", dx2, dx, B, D, H, W)
+        _lib.launch("b200_cross_scan_pack_bwd", dx2.device, dx2.data_ptr(), dx.data_ptr(), B, D, H, W, _lib.dtype_code(dx2.dtype))
         return dx
 
 
@@ -68,7 +60,7 @@ class CrossMergeFn(torch.autograd.Function):
         B, K, D, L = ys.shape
         assert K == 4 and L == H * W
         y = torch.empty((B, L, D), dtype=ys.dtype, device=ys.device)
-        _plane_op("b200_cross_merge", ys, y, B, D, H, W)
+        _lib.launch("b200_cross_merge", ys.device, ys.data_ptr(), y.data_ptr(), B, D, H, W, _lib.dtype_code(ys.dtype))
         ctx.hw = (H, W)
         return y
 
@@ -79,58 +71,9 @@ class CrossMergeFn(torch.autograd.Function):
         dy = dy.contiguous()
         B, L, D = dy.shape
         d2 = torch.empty((B, 2, D, L), dtype=dy.dtype, device=dy.device)
-        _plane_op("b200_cross_merge_bwd", dy, d2, B, D, H, W)
+        _lib.launch("b200_cross_merge_bwd", dy.device, dy.data_ptr(), d2.data_ptr(), B, D, H, W, _lib.dtype_code(dy.dtype))
         dys = d2.unsqueeze(2).expand(B, 2, 2, D, L).reshape(B, 4, D, L)
         return dys, None, None
-
-
-class ScanMergeFn(torch.autograd.Function):
-    """Four-direction selective scan + cross-merge in one autograd node.
-
-    x2 (B, 2, D, L) from CrossScanPackFn; delta (B, 4*D, L); A (4*D, N); Bs, Cs (B, 4, N, L);
-    Ds, delta_bias (4*D) -- all in the internal direction order.  Returns y (B, L, D) =
-    sum of the four directions at their image positions (== (B, H, W, D) flattened).
-    """
-
-    @staticmethod
-    @_no_autocast
-    def forward(ctx, x2, delta, A, Bs, Cs, Ds, delta_bias, H, W):
-        _lib.require_cuda(x2, delta, A, Bs, Cs, Ds, delta_bias)
-        B, two, D, L = x2.shape
-        assert two == 2 and L == H * W and delta.shape == (B, 4 * D, L)
-        x2 = x2.contiguous()
-        u = x2.view(B, 2 * D, L)
-        delta = delta if delta.stride(-1) == 1 else delta.contiguous()
-        Bs = Bs if Bs.stride(-1) == 1 else Bs.contiguous()
-        Cs = Cs if Cs.stride(-1) == 1 else Cs.contiguous()
-        if not (u.dtype == delta.dtype == Bs.dtype == Cs.dtype):
-            raise RuntimeError("ScanMergeFn: x2, delta, Bs, Cs must share a dtype")
-        A32, D32, b32 = _f32c(A), _f32c(Ds), _f32c(delta_bias)
-        need_grad = any(ctx.needs_input_grad)
-        ys, _, ckpt = launch_fwd(u, delta, A32, Bs, Cs, D32, None, b32, True, REV_MASK, 2, want_ckpt=need_grad)
-        y = torch.empty((B, L, D), dtype=ys.dtype, device=ys.device)
-        _plane_op("b200_cross_merge", ys, y, B, D, H, W)
-        if need_grad:
-            ctx.save_for_backward(u, delta, A32, Bs, Cs, D32, b32, ckpt)
-        ctx.hw = (H, W)
-        ctx.dtypes = (A.dtype, Ds.dtype, delta_bias.dtype)
-        return y
-
-    @staticmethod
-    @_no_autocast
-    def backward(ctx, dy):
-        u, delta, A32, Bs, Cs, D32, b32, ckpt = ctx.saved_tensors
-        H, W = ctx.hw
-        B, KD, L = delta.shape
-        D = KD // 4
-        dy = dy.contiguous().to(u.dtype)
-        d2 = torch.empty((B, 2 * D, L), dtype=dy.dtype, device=dy.device)
-        _plane_op("b200_cross_merge_bwd", dy, d2, B, D, H, W)
-        du, ddelta, dA, dB, dC, dD, dbias, _ = launch_bwd(u, delta, A32, Bs, Cs, D32, None, b32, True, ckpt, d2,
-                                                          REV_MASK, 2, 2, True, True)
-        dx2 = du.view(B, 2, 2, D, L).sum(2)
-        return (dx2, ddelta, dA.to(ctx.dtypes[0]), dB.to(Bs.dtype), dC.to(Cs.dtype), dD.to(ctx.dtypes[1]),
-                dbias.to(ctx.dtypes[2]), None, None)
 
 
 class _Tf32:
@@ -188,7 +131,6 @@ class SS2DCoreFn(torch.autograd.Function):
     @_no_autocast
     def forward(ctx, x, W_all, A, Ds, delta_bias, N, tf32):
         _lib.require_cuda(x, W_all, A, Ds, delta_bias)
-        lib = _lib.load()
         x = x.float().contiguous()
         B, D, H, W = x.shape
         L = H * W
@@ -202,21 +144,19 @@ class SS2DCoreFn(torch.autograd.Function):
         Lp = (L + 3) // 4 * 4
         x2 = torch.empty((2, D, B, Lp), dtype=torch.float32, device=dev) if Lp == L else torch.zeros((2, D, B, Lp), dtype=torch.float32, device=dev)
         strides = (Lp, D * B * Lp, B * Lp)                            # (batch, layout, row) element strides of x2
-        with torch.cuda.device(dev):
-            _lib.check(lib.b200_cross_scan_pack_strided(x.data_ptr(), x2.data_ptr(), *strides, B, D, H, W, _lib.stream_ptr(dev)),
-                       "b200_cross_scan_pack_strided")
+        _lib.launch("b200_cross_scan_pack_strided", dev, x.data_ptr(), x2.data_ptr(), *strides, B, D, H, W)
         Wm = W_all.detach().float().reshape(2, 2 * M, D).contiguous()
         with _Tf32(tf32):
             big = torch.bmm(Wm, x2.view(2, D, B * Lp))                 # (2, 2M, B*Lp)
         big4 = big.view(4, M, B, Lp).permute(2, 0, 1, 3)               # (B, 4, M, Lp) view
-        A32, D32, b32 = _f32c(A), _f32c(Ds), _f32c(delta_bias)
+        A32, D32, b32 = _lib.f32c(A), _lib.f32c(Ds), _lib.f32c(delta_bias)
         need_grad = any(ctx.needs_input_grad)
         ys, _, ckpt = launch_fwd(x2.permute(2, 0, 1, 3), big4[:, :, 2 * N:], A32, big4[:, :, :N], big4[:, :, N:2 * N], D32, None, b32,
                                  True, REV_MASK, 2, want_ckpt=need_grad, algo_len=L)
         if Lp != L:
             ys = ys[:, :, :L].contiguous()
         y = torch.empty((B, L, D), dtype=torch.float32, device=dev)
-        _plane_op("b200_cross_merge", ys, y, B, D, H, W)
+        _lib.launch("b200_cross_merge", dev, ys.data_ptr(), y.data_ptr(), B, D, H, W, _lib.dtype_code(ys.dtype))
         if need_grad:
             ctx.save_for_backward(x2, big, Wm, A32, D32, b32, ckpt)
         ctx.meta = (B, D, H, W, M, N, bool(tf32))
@@ -230,11 +170,10 @@ class SS2DCoreFn(torch.autograd.Function):
         B, D, H, W, M, N, tf32 = ctx.meta
         L = H * W
         Lp = x2.shape[-1]
-        lib = _lib.load()
         dev = dy.device
         dy = dy.contiguous().float()
         d2 = torch.empty((B, 2 * D, L), dtype=torch.float32, device=dev)
-        _plane_op("b200_cross_merge_bwd", dy, d2, B, D, H, W)
+        _lib.launch("b200_cross_merge_bwd", dev, dy.data_ptr(), d2.data_ptr(), B, D, H, W, _lib.dtype_code(dy.dtype))
         if Lp != L:
             d2 = torch.nn.functional.pad(d2, (0, Lp - L))              # zero upstream gradient at the pad steps
         big4 = big.view(4, M, B, Lp).permute(2, 0, 1, 3)
@@ -253,48 +192,13 @@ class SS2DCoreFn(torch.autograd.Function):
             dW = _weight_grad_splitk(g_big, x2m)                       # (2, 2M, D)
             gx2 = torch.bmm(Wm.transpose(1, 2), g_big)                 # (2, D, B*Lp)
         dx = torch.empty((B, D, H, W), dtype=torch.float32, device=dev)
-        with torch.cuda.device(dev):
-            _lib.check(lib.b200_cross_scan_unpack4(du.data_ptr(), gx2.data_ptr(), Lp, D * B * Lp, B * Lp, dx.data_ptr(), B, D, H, W,
-                                                   _lib.stream_ptr(dev)), "b200_cross_scan_unpack4")
+        _lib.launch("b200_cross_scan_unpack4", dev, du.data_ptr(), gx2.data_ptr(), Lp, D * B * Lp, B * Lp, dx.data_ptr(), B, D, H, W)
         wdt, adt, ddt, bdt = ctx.dtypes
         return dx, dW.view(4, M, D).to(wdt), dA.to(adt), dD.to(ddt), dbias.to(bdt), None, None
 
 
 def ss2d_core(x, W_all, A, Ds, delta_bias, N, tf32=False):
     return SS2DCoreFn.apply(x, W_all, A, Ds, delta_bias, N, tf32)
-
-
-class CrossScan4Fn(torch.autograd.Function):
-    """SSD twin of the cross-scan: x (B, C, H, W) fp32 (a channel slice of a wider NCHW tensor is read in place) ->
-    x4 (B, 4, C, L) in the reference's direction order (hw, wh, hw reversed, wh reversed; SSD/MedSSD.py:332-336)."""
-
-    @staticmethod
-    @_no_autocast
-    def forward(ctx, x):
-        _lib.require_cuda(x)
-        lib = _lib.load()
-        x = x.float()
-        B, C, H, W = x.shape
-        if not (x.stride(3) == 1 and x.stride(2) == W and x.stride(1) == H * W):
-            x = x.contiguous()
-        x4 = torch.empty((B, 4, C, H * W), dtype=torch.float32, device=x.device)
-        with torch.cuda.device(x.device):
-            _lib.check(lib.b200_cross_scan4(x.data_ptr(), x.stride(0), x4.data_ptr(), B, C, H, W, _lib.stream_ptr(x.device)), "b200_cross_scan4")
-        ctx.hw = (H, W)
-        return x4
-
-    @staticmethod
-    @_no_autocast
-    def backward(ctx, dx4):
-        lib = _lib.load()
-        H, W = ctx.hw
-        dx4 = dx4.float().contiguous()
-        B, _, C, _ = dx4.shape
-        dx = torch.empty((B, C, H, W), dtype=torch.float32, device=dx4.device)
-        with torch.cuda.device(dx4.device):
-            _lib.check(lib.b200_cross_scan4_bwd(dx4.data_ptr(), dx.data_ptr(), dx.stride(0), B, C, H, W, _lib.stream_ptr(dx4.device)),
-                       "b200_cross_scan4_bwd")
-        return dx
 
 
 class CrossScan4SplitFn(torch.autograd.Function):
@@ -306,41 +210,35 @@ class CrossScan4SplitFn(torch.autograd.Function):
     @_no_autocast
     def forward(ctx, x, *sizes):
         _lib.require_cuda(x)
-        lib = _lib.load()
         x = x.float()
         B, C, H, W = x.shape
         assert sum(sizes) == C
         if not (x.stride(3) == 1 and x.stride(2) == W and x.stride(1) == H * W):
             x = x.contiguous()
         outs, c0 = [], 0
-        with torch.cuda.device(x.device):
-            for n in sizes:
-                o = torch.empty((B, 4, n, H * W), dtype=torch.float32, device=x.device)
-                part = x[:, c0:c0 + n]
-                _lib.check(lib.b200_cross_scan4(part.data_ptr(), x.stride(0), o.data_ptr(), B, n, H, W, _lib.stream_ptr(x.device)), "b200_cross_scan4")
-                outs.append(o)
-                c0 += n
+        for n in sizes:
+            o = torch.empty((B, 4, n, H * W), dtype=torch.float32, device=x.device)
+            _lib.launch("b200_cross_scan4", x.device, x[:, c0:c0 + n].data_ptr(), x.stride(0), o.data_ptr(), B, n, H, W)
+            outs.append(o)
+            c0 += n
         ctx.meta = (B, C, H, W, tuple(sizes))
         return tuple(outs)
 
     @staticmethod
     @_no_autocast
     def backward(ctx, *douts):
-        lib = _lib.load()
         B, C, H, W, sizes = ctx.meta
         dev = next(g for g in douts if g is not None).device
         dx = torch.empty((B, C, H, W), dtype=torch.float32, device=dev)
         c0 = 0
-        with torch.cuda.device(dev):
-            for n, g in zip(sizes, douts):
-                part = dx[:, c0:c0 + n]
-                if g is None:
-                    part.zero_()
-                else:
-                    g = g.float().contiguous()
-                    _lib.check(lib.b200_cross_scan4_bwd(g.data_ptr(), part.data_ptr(), dx.stride(0), B, n, H, W, _lib.stream_ptr(dev)),
-                               "b200_cross_scan4_bwd")
-                c0 += n
+        for n, g in zip(sizes, douts):
+            part = dx[:, c0:c0 + n]
+            if g is None:
+                part.zero_()
+            else:
+                g = g.float().contiguous()
+                _lib.launch("b200_cross_scan4_bwd", dev, g.data_ptr(), part.data_ptr(), dx.stride(0), B, n, H, W)
+            c0 += n
         return (dx,) + (None,) * len(sizes)
 
 
@@ -356,30 +254,28 @@ class SsdMerge4Fn(torch.autograd.Function):
     @_no_autocast
     def forward(ctx, y, H, W):
         _lib.require_cuda(y)
-        lib = _lib.load()
         y = y.float().contiguous()
         B, L, K, d = y.shape
         assert K == 4 and L == H * W
         out = torch.empty((B, L, d), dtype=torch.float32, device=y.device)
-        with torch.cuda.device(y.device):
-            _lib.check(lib.b200_ssd_merge4(y.data_ptr(), out.data_ptr(), B, d, H, W, _lib.stream_ptr(y.device)), "b200_ssd_merge4")
+        _lib.launch("b200_ssd_merge4", y.device, y.data_ptr(), out.data_ptr(), B, d, H, W)
         ctx.meta = (B, L, d, H, W)
         return out
 
     @staticmethod
     @_no_autocast
     def backward(ctx, dout):
-        lib = _lib.load()
         B, L, d, H, W = ctx.meta
         dout = dout.float().contiguous()
         dy = torch.empty((B, L, 4, d), dtype=torch.float32, device=dout.device)
-        with torch.cuda.device(dout.device):
-            _lib.check(lib.b200_ssd_merge4_bwd(dout.data_ptr(), dy.data_ptr(), B, d, H, W, _lib.stream_ptr(dout.device)), "b200_ssd_merge4_bwd")
+        _lib.launch("b200_ssd_merge4_bwd", dout.device, dout.data_ptr(), dy.data_ptr(), B, d, H, W)
         return dy, None, None
 
 
 def cross_scan4(x):
-    return CrossScan4Fn.apply(x)
+    """SSD twin of the cross-scan: x (B, C, H, W) fp32 (a channel slice of a wider NCHW tensor is read in place) ->
+    x4 (B, 4, C, L) in the reference's direction order (hw, wh, hw reversed, wh reversed; SSD/MedSSD.py:332-336)."""
+    return cross_scan4_split(x, (x.shape[1],))[0]
 
 
 def ssd_merge4(y, H, W):
@@ -392,7 +288,3 @@ def cross_scan_pack(x):
 
 def cross_merge(ys, H, W):
     return CrossMergeFn.apply(ys, H, W)
-
-
-def scan_merge(x2, delta, A, Bs, Cs, Ds, delta_bias, H, W):
-    return ScanMergeFn.apply(x2, delta, A, Bs, Cs, Ds, delta_bias, H, W)

@@ -14,8 +14,9 @@ import torch
 
 import torch.nn as nn
 
+from . import _lib
 from ._lib import no_autocast as _no_autocast
-from .ss2d import SS2D, split_halves
+from .ss2d import SS2D, LnGateFn, layer_norm_rows, split_halves
 from .ss2d_ssd import SS2D_with_SSD
 
 
@@ -42,7 +43,6 @@ def _layer_norm(x, norm):
     replaces PyTorch's gamma/beta reduction (3.9 % of the step at 200 K rows x 96 channels).  Output dtype follows
     autocast like F.layer_norm's consumer would see it (fp32 without autocast)."""
     if isinstance(norm, nn.LayerNorm) and norm.elementwise_affine and x.shape[-1] <= 1024 and x.dtype in (torch.float32, torch.bfloat16):
-        from .ss2d import LnGateFn
         x = x.contiguous()   # rows contiguous (no-op when already so); fp32 or bf16 rows are read as they are
         return LnGateFn.apply(x, None, norm.weight, norm.bias, norm.eps, torch.float32)
     return norm(x)
@@ -70,28 +70,20 @@ class PatchMergeGatherFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, x):
-        from . import _lib
         _lib.require_cuda(x)
-        lib = _lib.load()
         x = x.contiguous()
         B, H, W, C = x.shape
         out = torch.empty((B, H // 2, W // 2, 4 * C), dtype=x.dtype, device=x.device)
-        with torch.cuda.device(x.device):
-            _lib.check(lib.b200_patch_merge(x.data_ptr(), out.data_ptr(), B, H, W, C * x.element_size(), 0, _lib.stream_ptr(x.device)),
-                       "b200_patch_merge")
+        _lib.launch("b200_patch_merge", x.device, x.data_ptr(), out.data_ptr(), B, H, W, C * x.element_size(), 0)
         ctx.shape = (B, H, W, C)
         return out
 
     @staticmethod
     def backward(ctx, dout):
-        from . import _lib
-        lib = _lib.load()
         B, H, W, C = ctx.shape
         dout = dout.contiguous()
         dx = torch.empty((B, H, W, C), dtype=dout.dtype, device=dout.device)
-        with torch.cuda.device(dout.device):
-            _lib.check(lib.b200_patch_merge(dout.data_ptr(), dx.data_ptr(), B, H, W, C * dout.element_size(), 1, _lib.stream_ptr(dout.device)),
-                       "b200_patch_merge")
+        _lib.launch("b200_patch_merge", dout.device, dout.data_ptr(), dx.data_ptr(), B, H, W, C * dout.element_size(), 1)
         return dx
 
 
@@ -129,9 +121,7 @@ class ShuffleCatAddFn(torch.autograd.Function):
     @staticmethod
     @_no_autocast
     def forward(ctx, left, x, inp):
-        from . import _lib
         _lib.require_cuda(left, x, inp)
-        lib = _lib.load()
         B, c, H, W = left.shape
         cl = left.is_contiguous(memory_format=torch.channels_last) and not left.is_contiguous()
         if not cl:
@@ -140,25 +130,20 @@ class ShuffleCatAddFn(torch.autograd.Function):
             inp = inp.float()                                  # torch would promote the sum to fp32
         x, inp = x.to(left.dtype).contiguous(), inp.contiguous()
         out = torch.empty((B, H, W, 2 * c), dtype=inp.dtype, device=inp.device)
-        with torch.cuda.device(inp.device):
-            _lib.check(lib.b200_shuffle_cat_add_fwd(left.data_ptr(), int(cl), x.data_ptr(), _lib.dtype_code(left.dtype), inp.data_ptr(),
-                                                    out.data_ptr(), _lib.dtype_code(inp.dtype), B, c, H * W, _lib.stream_ptr(inp.device)),
-                       "b200_shuffle_cat_add_fwd")
+        _lib.launch("b200_shuffle_cat_add_fwd", inp.device, left.data_ptr(), int(cl), x.data_ptr(), _lib.dtype_code(left.dtype),
+                    inp.data_ptr(), out.data_ptr(), _lib.dtype_code(inp.dtype), B, c, H * W)
         ctx.meta = (B, c, H, W, left.dtype, cl, inp.dtype)
         return out
 
     @staticmethod
     @_no_autocast
     def backward(ctx, dout):
-        from . import _lib
-        lib = _lib.load()
         B, c, H, W, ldt, cl, iodt = ctx.meta
         dout = dout.to(iodt).contiguous()
         dleft = torch.empty((B, c, H, W), dtype=ldt, device=dout.device, memory_format=torch.channels_last if cl else torch.contiguous_format)
         dx = torch.empty((B, H, W, c), dtype=ldt, device=dout.device)
-        with torch.cuda.device(dout.device):
-            _lib.check(lib.b200_shuffle_cat_add_bwd(dout.data_ptr(), _lib.dtype_code(iodt), dleft.data_ptr(), int(cl), dx.data_ptr(),
-                                                    _lib.dtype_code(ldt), B, c, H * W, _lib.stream_ptr(dout.device)), "b200_shuffle_cat_add_bwd")
+        _lib.launch("b200_shuffle_cat_add_bwd", dout.device, dout.data_ptr(), _lib.dtype_code(iodt), dleft.data_ptr(), int(cl), dx.data_ptr(),
+                    _lib.dtype_code(ldt), B, c, H * W)
         return dleft, dx, dout
 
 
@@ -215,7 +200,6 @@ class SS_Conv_SSM(nn.Module):
         return self.conv33conv33conv11(left)
 
     def forward(self, input):
-        from . import _lib
         _lib.require_cuda(input)                           # no CPU path: oracle/cpu_path.py holds the eager CPU tree
         left, right = split_halves(input)
         side = None
@@ -226,7 +210,6 @@ class SS_Conv_SSM(nn.Module):
             with torch.cuda.stream(side):
                 left = self._conv_branch(left)
         if right.dtype in (torch.float32, torch.bfloat16) and isinstance(self.ln_1, nn.LayerNorm) and right.shape[-1] <= 1024:
-            from .ss2d import layer_norm_rows
             normed = layer_norm_rows(right, self.ln_1)     # pre-norm, the right half read in place (csrc/lngate.cu)
         else:
             normed = self.ln_1(right)

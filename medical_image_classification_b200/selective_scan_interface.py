@@ -42,12 +42,6 @@ def _last_contig(t):
     return t if t is None or t.stride(-1) == 1 else t.contiguous()
 
 
-def _f32c(t):
-    if t is None:
-        return None
-    return t.detach().to(torch.float32).contiguous()
-
-
 def _row_strides(t, rpg):
     """(batch, group, row) element strides of an activation given as (B, dim, L) or as a (B, G', rows, L) view."""
     if t.dim() == 4:
@@ -101,13 +95,12 @@ def launch_fwd(u, delta, A32, Bm, Cm, D32, z, bias32, delta_softplus, rev_mask=0
                want_ckpt=False, want_last_state=False, algo_len=None):
     """One b200_sscan_fwd call on prepared tensors (last stride 1, B/C 4-D, A/D/bias fp32 contiguous).
     Returns (out, last_state | None, ckpt | None)."""
-    lib = _lib.load()
     batch, L, dim = delta.shape[0], delta.shape[-1], A32.shape[0]
     G, N = Bm.shape[1], Bm.shape[2]
     out = torch.empty((batch, dim, L), dtype=u.dtype, device=u.device)
     ckpt = None
     if want_ckpt:
-        nbytes = lib.b200_sscan_ckpt_bytes(batch, dim, L, N, G, CKPT_EVERY)
+        nbytes = _lib.load().b200_sscan_ckpt_bytes(batch, dim, L, N, G, CKPT_EVERY)
         ckpt = torch.empty(nbytes // 4, dtype=torch.float32, device=u.device)
     last_state = torch.empty((batch, dim, N), dtype=torch.float32, device=u.device) if want_last_state else None
     p = _lib.SScanFwdParams()
@@ -118,7 +111,7 @@ def launch_fwd(u, delta, A32, Bm, Cm, D32, z, bias32, delta_softplus, rev_mask=0
     prof = _profiler
     with torch.cuda.device(u.device):
         tok = prof.begin() if prof is not None else None
-        _lib.check(lib.b200_sscan_fwd(C.byref(p), _lib.stream_ptr(u.device)), "b200_sscan_fwd")
+        _lib.launch("b200_sscan_fwd", u.device, C.byref(p))
         if prof is not None:
             prof.end(tok, "fwd", u, delta, Bm, algo_len)
     return out, last_state, ckpt
@@ -130,7 +123,6 @@ def launch_bwd(u, delta, A32, Bm, Cm, D32, z, bias32, delta_softplus, ckpt, dout
     Returns du (batch, dim, L), ddelta, dA, dB, dC (fp32), dD, ddelta_bias, dz.
     ddelta (batch, G, rows per group, L) and dB, dC (batch, G, N, L; fp32, ZERO-FILLED by the caller) may be passed as
     views into a wider buffer (last stride 1); they are then written / accumulated in place."""
-    lib = _lib.load()
     batch, L, dim = delta.shape[0], delta.shape[-1], A32.shape[0]
     G, N = Bm.shape[1], Bm.shape[2]
     rpg = dim // G
@@ -164,7 +156,7 @@ def launch_bwd(u, delta, A32, Bm, Cm, D32, z, bias32, delta_softplus, ckpt, dout
     prof = _profiler
     with torch.cuda.device(dev):
         tok = prof.begin() if prof is not None else None
-        _lib.check(lib.b200_sscan_bwd(C.byref(q), _lib.stream_ptr(dev)), "b200_sscan_bwd")
+        _lib.launch("b200_sscan_bwd", dev, C.byref(q))
         if prof is not None:
             prof.end(tok, "bwd", u, delta, Bm, algo_len)
     return du, ddelta, dA, dB, dC, dD, dbias, dz
@@ -193,7 +185,7 @@ class SelectiveScanFn(torch.autograd.Function):
         if Bm.shape != Cm.shape or Bm.shape[0] != batch or Bm.shape[3] != L or dim % G != 0 or A.shape[1] != N:
             raise RuntimeError(f"selective_scan: B {tuple(B.shape)} / C {tuple(C.shape)} do not match "
                                f"delta {tuple(delta.shape)} and A {tuple(A.shape)}")
-        A32, D32, bias32 = _f32c(A), _f32c(D), _f32c(delta_bias)
+        A32, D32, bias32 = _lib.f32c(A), _lib.f32c(D), _lib.f32c(delta_bias)
         need_grad = any(ctx.needs_input_grad)
         out, last_state, ckpt = launch_fwd(u, delta, A32, Bm, Cm, D32, z, bias32, delta_softplus, rev_mask,
                                            u_group_div, want_ckpt=need_grad, want_last_state=return_last_state)

@@ -22,54 +22,8 @@ import torch.nn.functional as F
 
 from . import _lib
 from ._lib import no_autocast as _no_autocast
-from .cross import cross_scan_pack, scan_merge, ss2d_core  # noqa: F401
+from .cross import ss2d_core
 from .selective_scan_interface import selective_scan_fn
-
-
-class _tf32_matmul:
-    """Context: run fp32 matmuls on the TF32 tensor-core path (restores the global flag on exit)."""
-
-    def __init__(self, on: bool):
-        self.on = on
-
-    def __enter__(self):
-        self.prev = torch.backends.cuda.matmul.allow_tf32
-        if self.on:
-            torch.backends.cuda.matmul.allow_tf32 = True
-
-    def __exit__(self, *exc):
-        torch.backends.cuda.matmul.allow_tf32 = self.prev
-
-
-class _ProjFn(torch.autograd.Function):
-    """out = W @ X for the x_proj / dt_proj contractions (MedMamba.py:397-400) with the precision fixed at call time
-    for BOTH passes: `tf32=True` is used under autocast, where the reference runs these einsums in bf16 -- TF32 on the
-    fp32 operands keeps more mantissa (10 bits vs 8) and needs no casts; `tf32=False` is exact fp32 (parity tests)."""
-
-    @staticmethod
-    @_no_autocast
-    def forward(ctx, W, X, tf32):
-        ctx.save_for_backward(W, X)
-        ctx.tf32 = bool(tf32)
-        with _tf32_matmul(ctx.tf32):
-            return torch.matmul(W, X)
-
-    @staticmethod
-    @_no_autocast
-    def backward(ctx, g):
-        W, X = ctx.saved_tensors
-        dW = dX = None
-        with _tf32_matmul(ctx.tf32):
-            if ctx.needs_input_grad[0]:
-                dW = torch.matmul(g, X.transpose(-1, -2))
-                while dW.dim() > W.dim():        # W was broadcast over leading (batch) dimensions
-                    dW = dW.sum(0)
-                for ax, (a, b_) in enumerate(zip(dW.shape, W.shape)):
-                    if a != b_:
-                        dW = dW.sum(ax, keepdim=True)
-            if ctx.needs_input_grad[1]:
-                dX = torch.matmul(W.transpose(-1, -2), g)
-        return dW, dX, None
 
 
 def _rows_view(t, D):
@@ -114,9 +68,7 @@ class LnGateFn(torch.autograd.Function):
     @staticmethod
     @_no_autocast
     def forward(ctx, y, z, weight, bias, eps, out_dtype):
-        from . import _lib
         _lib.require_cuda(y, z, weight, bias)
-        lib = _lib.load()
         D = y.shape[-1]
         if y.dtype != torch.float32 and not (y.dtype == torch.bfloat16 and z is None):
             y = y.float()
@@ -132,10 +84,8 @@ class LnGateFn(torch.autograd.Function):
         mean = torch.empty(rows, dtype=torch.float32, device=y.device)
         rstd = torch.empty(rows, dtype=torch.float32, device=y.device)
         zcode = _lib.dtype_code(z2.dtype) if z2 is not None else 0
-        with torch.cuda.device(y.device):
-            _lib.check(lib.b200_ln_gate_fwd(y2.data_ptr(), _lib.dtype_code(y2.dtype), ys, _lib.ptr(z2), zs, zcode, w32.data_ptr(), b32.data_ptr(), out.data_ptr(),
-                                            _lib.dtype_code(out_dtype), mean.data_ptr(), rstd.data_ptr(), rows, D, float(eps),
-                                            _lib.stream_ptr(y.device)), "b200_ln_gate_fwd")
+        _lib.launch("b200_ln_gate_fwd", y.device, y2.data_ptr(), _lib.dtype_code(y2.dtype), ys, _lib.ptr(z2), zs, zcode, w32.data_ptr(),
+                    b32.data_ptr(), out.data_ptr(), _lib.dtype_code(out_dtype), mean.data_ptr(), rstd.data_ptr(), rows, D, float(eps))
         ctx.save_for_backward(y2, z2, w32, b32, mean, rstd)
         ctx.ys, ctx.zs, ctx.shape, ctx.zshape, ctx.rows = ys, zs, y.shape, (z.shape if z is not None else None), rows
         ctx.wdtype, ctx.bdtype = weight.dtype, bias.dtype
@@ -144,21 +94,18 @@ class LnGateFn(torch.autograd.Function):
     @staticmethod
     @_no_autocast
     def backward(ctx, dout):
-        from . import _lib
-        lib = _lib.load()
         y2, z2, w32, b32, mean, rstd = ctx.saved_tensors
         rows, D = ctx.rows, ctx.shape[-1]
         dout = dout.reshape(rows, D).contiguous()
         dev = dout.device
         dy = torch.empty((rows, D), dtype=y2.dtype, device=dev)
         dz = torch.empty((rows, D), dtype=z2.dtype, device=dev) if z2 is not None else None
-        grid = lib.b200_ln_gate_grid(rows)
+        grid = _lib.load().b200_ln_gate_grid(rows)
         part = torch.empty((2, grid, D), dtype=torch.float32, device=dev)
         zcode = _lib.dtype_code(z2.dtype) if z2 is not None else 0
-        with torch.cuda.device(dev):
-            _lib.check(lib.b200_ln_gate_bwd(dout.data_ptr(), y2.data_ptr(), _lib.dtype_code(y2.dtype), ctx.ys, _lib.ptr(z2), ctx.zs, zcode, w32.data_ptr(), b32.data_ptr(),
-                                            _lib.dtype_code(dout.dtype), mean.data_ptr(), rstd.data_ptr(), dy.data_ptr(), _lib.ptr(dz),
-                                            part[0].data_ptr(), part[1].data_ptr(), rows, D, _lib.stream_ptr(dev)), "b200_ln_gate_bwd")
+        _lib.launch("b200_ln_gate_bwd", dev, dout.data_ptr(), y2.data_ptr(), _lib.dtype_code(y2.dtype), ctx.ys, _lib.ptr(z2), ctx.zs, zcode,
+                    w32.data_ptr(), b32.data_ptr(), _lib.dtype_code(dout.dtype), mean.data_ptr(), rstd.data_ptr(), dy.data_ptr(), _lib.ptr(dz),
+                    part[0].data_ptr(), part[1].data_ptr(), rows, D)
         dwb = part.sum(1)
         return (dy.view(ctx.shape), dz.view(ctx.zshape) if dz is not None else None, dwb[0].to(ctx.wdtype), dwb[1].to(ctx.bdtype),
                 None, None)
@@ -171,9 +118,7 @@ class DwConvSiluFn(torch.autograd.Function):
     @staticmethod
     @_no_autocast
     def forward(ctx, xin, weight, bias):
-        from . import _lib
         _lib.require_cuda(xin, weight, bias)
-        lib = _lib.load()
         B, H, W, D = xin.shape
         ok = xin.stride(3) == 1 and xin.stride(1) == W * xin.stride(2) and xin.stride(0) == H * xin.stride(1)
         if not ok or xin.dtype not in (torch.float32, torch.bfloat16):
@@ -181,9 +126,8 @@ class DwConvSiluFn(torch.autograd.Function):
         w32 = weight.detach().float().reshape(D, 9).contiguous()
         b32 = bias.detach().float().contiguous() if bias is not None else None
         out = torch.empty((B, D, H, W), dtype=torch.float32, device=xin.device)
-        with torch.cuda.device(xin.device):
-            _lib.check(lib.b200_dwconv_silu_fwd(xin.data_ptr(), xin.stride(2), _lib.dtype_code(xin.dtype), w32.data_ptr(), _lib.ptr(b32),
-                                                out.data_ptr(), B, D, H, W, _lib.stream_ptr(xin.device)), "b200_dwconv_silu_fwd")
+        _lib.launch("b200_dwconv_silu_fwd", xin.device, xin.data_ptr(), xin.stride(2), _lib.dtype_code(xin.dtype), w32.data_ptr(),
+                    _lib.ptr(b32), out.data_ptr(), B, D, H, W)
         ctx.save_for_backward(xin, w32, b32)
         ctx.wshape, ctx.wdtype = weight.shape, weight.dtype
         ctx.bdtype = bias.dtype if bias is not None else None
@@ -192,18 +136,14 @@ class DwConvSiluFn(torch.autograd.Function):
     @staticmethod
     @_no_autocast
     def backward(ctx, g):
-        from . import _lib
-        lib = _lib.load()
         xin, w32, b32 = ctx.saved_tensors
         B, H, W, D = xin.shape
         g = g.float().contiguous()
         dxin = torch.empty((B, H, W, D), dtype=xin.dtype, device=xin.device)
         acc_w = torch.zeros((D * 9 + D,), dtype=torch.float32, device=xin.device)   # weight taps | bias: one memset
         dw_buf, db_buf = acc_w[: D * 9], acc_w[D * 9:]
-        with torch.cuda.device(xin.device):
-            _lib.check(lib.b200_dwconv_silu_bwd(g.data_ptr(), xin.data_ptr(), xin.stride(2), _lib.dtype_code(xin.dtype), w32.data_ptr(),
-                                                _lib.ptr(b32), dxin.data_ptr(), dw_buf.data_ptr(), db_buf.data_ptr(), B, D, H, W,
-                                                _lib.stream_ptr(xin.device)), "b200_dwconv_silu_bwd")
+        _lib.launch("b200_dwconv_silu_bwd", xin.device, g.data_ptr(), xin.data_ptr(), xin.stride(2), _lib.dtype_code(xin.dtype),
+                    w32.data_ptr(), _lib.ptr(b32), dxin.data_ptr(), dw_buf.data_ptr(), db_buf.data_ptr(), B, D, H, W)
         dweight = dw_buf.view(ctx.wshape).to(ctx.wdtype)
         dbias = db_buf.to(ctx.bdtype) if ctx.bdtype is not None else None
         return dxin, dweight, dbias

@@ -76,17 +76,9 @@ def _fill_fwd(p, x, dt, A, Bm, Cm, D, dt_bias, chunk_size, dt_softplus, dt_limit
     p.D, p.dt_bias, p.initial_states = _lib.ptr(D), _lib.ptr(dt_bias), _lib.ptr(initial_states)
 
 
-def _f32c(t):
-    return None if t is None else t.detach().to(torch.float32).contiguous()
-
-
 def _empty_like_layout(t):
     """fp32 tensor of t's shape with t's strides when t is dense (any dimension order), contiguous otherwise."""
-    expect, dense = 1, True
-    for size, stride in sorted(((sz, st) for sz, st in zip(t.shape, t.stride()) if sz != 1), key=lambda e: e[1]):
-        dense = dense and stride == expect
-        expect *= size
-    if dense and all(st > 0 for sz, st in zip(t.shape, t.stride()) if sz != 1):
+    if _lib.is_dense(t):
         return torch.empty_strided(t.shape, t.stride(), dtype=torch.float32, device=t.device)
     return torch.empty(t.shape, dtype=torch.float32, device=t.device)
 
@@ -95,15 +87,14 @@ class SsdChunkScanFn(torch.autograd.Function):
     @staticmethod
     @_no_autocast
     def forward(ctx, x, dt, A, B, C, D, dt_bias, initial_states, chunk_size, dt_softplus, dt_limit, return_final_states, prec):
-        lib = _lib.load()
         batch, L, H, P = x.shape
         G, N = B.shape[2], B.shape[3]
         dev = x.device
         dt_, B_, C_ = dt.to(x.dtype), B.to(x.dtype), C.to(x.dtype)
-        A32, D32, bias32, init32 = _f32c(A), _f32c(D), _f32c(dt_bias), _f32c(initial_states)
+        A32, D32, bias32, init32 = _lib.f32c(A), _lib.f32c(D), _lib.f32c(dt_bias), _lib.f32c(initial_states)
         out = torch.empty((batch, L, H, P), dtype=x.dtype, device=dev)
         fin = torch.empty((batch, H, P, N), dtype=torch.float32, device=dev) if return_final_states else None
-        nbytes = lib.b200_ssd_workspace_bytes(batch, L, H, P, G, N, chunk_size)
+        nbytes = _lib.load().b200_ssd_workspace_bytes(batch, L, H, P, G, N, chunk_size)
         ws = torch.empty(nbytes // 4, dtype=torch.float32, device=dev)
         p = _lib.SsdFwdParams()
         _fill_fwd(p, x, dt_, A32, B_, C_, D32, bias32, chunk_size, dt_softplus, dt_limit, init32, prec)
@@ -112,7 +103,7 @@ class SsdChunkScanFn(torch.autograd.Function):
         prof = _profiler
         with torch.cuda.device(dev):
             tok = prof.begin() if prof is not None else None
-            _lib.check(lib.b200_ssd_fwd(ctypes.byref(p), _lib.stream_ptr(dev)), "b200_ssd_fwd")
+            _lib.launch("b200_ssd_fwd", dev, ctypes.byref(p))
             if prof is not None:
                 prof.end(tok, "fwd", (batch, L, H, P, G, N, chunk_size, prec))
         ctx.save_for_backward(x, dt_, A32, B_, C_, D32, bias32, init32, out, ws)
@@ -127,7 +118,6 @@ class SsdChunkScanFn(torch.autograd.Function):
     @staticmethod
     @_no_autocast
     def backward(ctx, dout, *unused):
-        lib = _lib.load()
         x, dt_, A32, B_, C_, D32, bias32, init32, out, ws = ctx.saved_tensors
         chunk_size, dt_softplus, dt_limit, precision = ctx.cfg
         batch, L, H, P = x.shape
@@ -140,7 +130,7 @@ class SsdChunkScanFn(torch.autograd.Function):
         dA = torch.zeros(H, dtype=torch.float32, device=dev)
         dD = torch.zeros(H, dtype=torch.float32, device=dev) if D32 is not None else None
         dbias = torch.zeros(H, dtype=torch.float32, device=dev) if bias32 is not None else None
-        nbytes = lib.b200_ssd_bwd_scratch_bytes(batch, L, H, P, G, N, chunk_size)
+        nbytes = _lib.load().b200_ssd_bwd_scratch_bytes(batch, L, H, P, G, N, chunk_size)
         scratch = torch.empty(nbytes // 4, dtype=torch.float32, device=dev)
         q = _lib.SsdBwdParams()
         _fill_fwd(q.f, x, dt_, A32, B_, C_, D32, bias32, chunk_size, dt_softplus, dt_limit, init32, precision)
@@ -154,7 +144,7 @@ class SsdChunkScanFn(torch.autograd.Function):
         prof = _profiler
         with torch.cuda.device(dev):
             tok = prof.begin() if prof is not None else None
-            _lib.check(lib.b200_ssd_bwd(ctypes.byref(q), _lib.stream_ptr(dev)), "b200_ssd_bwd")
+            _lib.launch("b200_ssd_bwd", dev, ctypes.byref(q))
             if prof is not None:
                 prof.end(tok, "bwd", (batch, L, H, P, G, N, chunk_size, precision))
         t_dt, t_A, t_B, t_C, t_D, t_bias = ctx.dtypes
@@ -228,7 +218,6 @@ class RmsNormGatedFn(torch.autograd.Function):
     @staticmethod
     @_no_autocast
     def forward(ctx, x, z, w, eps):
-        lib = _lib.load()
         _lib.require_cuda(x, z, w)
         shape = x.shape
         dim = shape[-1]
@@ -238,9 +227,8 @@ class RmsNormGatedFn(torch.autograd.Function):
         rows = x2.shape[0]
         y = torch.empty_like(x2)
         rstd = torch.empty(rows, dtype=torch.float32, device=x.device)
-        with torch.cuda.device(x.device):
-            _lib.check(lib.b200_rmsnorm_gated_fwd(x2.data_ptr(), z2.data_ptr(), w32.data_ptr(), y.data_ptr(), rstd.data_ptr(),
-                                                  rows, dim, float(eps), _lib.stream_ptr(x.device)), "b200_rmsnorm_gated_fwd")
+        _lib.launch("b200_rmsnorm_gated_fwd", x.device, x2.data_ptr(), z2.data_ptr(), w32.data_ptr(), y.data_ptr(), rstd.data_ptr(),
+                    rows, dim, float(eps))
         ctx.save_for_backward(x2, z2, w32, rstd)
         ctx.meta = (shape, x.dtype, z.dtype, w.dtype)
         return y.view(shape).to(x.dtype)
@@ -248,7 +236,6 @@ class RmsNormGatedFn(torch.autograd.Function):
     @staticmethod
     @_no_autocast
     def backward(ctx, dy):
-        lib = _lib.load()
         x2, z2, w32, rstd = ctx.saved_tensors
         shape, xdt, zdt, wdt = ctx.meta
         rows, dim = x2.shape
@@ -257,10 +244,8 @@ class RmsNormGatedFn(torch.autograd.Function):
         dz = torch.empty_like(x2)
         nblk = int(min(rows, 592))
         dwp = torch.empty((nblk, dim), dtype=torch.float32, device=x2.device)
-        with torch.cuda.device(x2.device):
-            _lib.check(lib.b200_rmsnorm_gated_bwd(x2.data_ptr(), z2.data_ptr(), w32.data_ptr(), rstd.data_ptr(), dy2.data_ptr(),
-                                                  dx.data_ptr(), dz.data_ptr(), dwp.data_ptr(), nblk, rows, dim,
-                                                  _lib.stream_ptr(x2.device)), "b200_rmsnorm_gated_bwd")
+        _lib.launch("b200_rmsnorm_gated_bwd", x2.device, x2.data_ptr(), z2.data_ptr(), w32.data_ptr(), rstd.data_ptr(), dy2.data_ptr(),
+                    dx.data_ptr(), dz.data_ptr(), dwp.data_ptr(), nblk, rows, dim)
         return dx.view(shape).to(xdt), dz.view(shape).to(zdt), dwp.sum(0).to(wdt), None
 
 

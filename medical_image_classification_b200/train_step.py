@@ -38,15 +38,7 @@ from __future__ import annotations
 import torch
 import torch.distributed as dist
 
-
-def _dense(t) -> bool:
-    """True when the tensor's elements fill one contiguous block exactly once (any dimension order, e.g. channels_last)."""
-    expect = 1
-    for size, stride in sorted(((sz, st) for sz, st in zip(t.shape, t.stride()) if sz != 1), key=lambda e: e[1]):
-        if stride != expect:
-            return False
-        expect *= size
-    return True
+from ._lib import is_dense as _dense
 
 
 class FlatGradSync:

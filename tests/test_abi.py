@@ -1,6 +1,6 @@
 """CPU-side checks of the drop-in boundary: the C-ABI library builds/loads, exports every symbol
-include/b200_ssm.h declares, the ctypes structs match the C layout, and the product refuses to run
-without CUDA (no CPU fallback).  No compute calls here."""
+include/b200_ssm.h declares, the ctypes binding gives each one the argument and return types of its prototype, the
+ctypes structs match the C layout, and the product refuses to run without CUDA (no CPU fallback).  No compute calls here."""
 import ctypes
 import os
 import re
@@ -24,6 +24,49 @@ def test_library_loads_and_exports_every_declared_symbol():
     for name in declared:
         assert hasattr(lib, name), name
     assert lib.b200_version() >= 1
+
+
+def _header_prototypes():
+    """[(name, return type, [parameter types])] of every b200_* function include/b200_ssm.h declares, in order."""
+    src = open(os.path.join(ROOT, "include", "b200_ssm.h")).read()
+    src = re.sub(r"/\*.*?\*/", " ", src, flags=re.S)
+    src = re.sub(r"//[^\n]*|^\s*#[^\n]*", " ", src, flags=re.M)
+    protos = []
+    for stmt in src.split(";"):
+        m = re.fullmatch(r"(.*?)\b(b200_\w+)\s*\((.*)\)", re.split(r"[{}]", stmt)[-1].strip(), flags=re.S)
+        if m is None:
+            continue
+        params = [" ".join(p.split()) for p in m.group(3).split(",")]
+        if params == ["void"]:
+            params = []
+        # drop each parameter's name: what remains is its type, with the pointer stars kept
+        types = [re.fullmatch(r"(.*?[\s*])\w+", p).group(1).replace(" *", "*").strip() for p in params]
+        protos.append((m.group(2), " ".join(m.group(1).split()).replace(" *", "*"), types))
+    return protos
+
+
+def test_binding_table_matches_header_prototypes():
+    """Every entry of _lib.SIGNATURES has the arity, parameter types and return type of its prototype in the header: a
+    mistyped int64_t stride or float would otherwise be converted silently and read as a wrong argument by the kernel."""
+    structs = {"b200_sscan_fwd_params": _lib.SScanFwdParams, "b200_sscan_bwd_params": _lib.SScanBwdParams,
+               "b200_ssd_fwd_params": _lib.SsdFwdParams, "b200_ssd_bwd_params": _lib.SsdBwdParams}
+    scalars = {"int32_t": ctypes.c_int32, "int64_t": ctypes.c_int64, "float": ctypes.c_float, "b200_stream_t": ctypes.c_void_p}
+    returns = {"int": ctypes.c_int, "size_t": ctypes.c_size_t, "const char*": ctypes.c_char_p}
+
+    def param_type(t):
+        if t.endswith("*"):
+            base = t.rstrip("*").replace("const ", "").strip()
+            return ctypes.POINTER(structs[base]) if base in structs else ctypes.c_void_p
+        return scalars[t]
+
+    protos = _header_prototypes()
+    assert [name for name, _, _ in protos] == list(_lib.SIGNATURES)
+    for name, ret, params in protos:
+        restype, argtypes = _lib.SIGNATURES[name]
+        assert restype is returns[ret], (name, ret, restype)
+        assert len(argtypes) == len(params), (name, params, argtypes)
+        for i, (t, declared) in enumerate(zip(params, argtypes)):
+            assert declared is param_type(t), (name, i, t, declared)
 
 
 def test_struct_layouts_match():
