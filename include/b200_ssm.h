@@ -275,6 +275,30 @@ int b200_rmsnorm_gated_bwd(const float* x, const float* z, const float* w, const
                            int32_t dw_rows, int64_t rows, int32_t dim, b200_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Gated RMSNorm with groups: every configuration of mamba_ssm's layernorm_gated RMSNorm / rmsnorm_fn (mamba_ssm 2.2.2,
+ * rms_norm_ref), which SS2D_with_SSD builds as RMSNorm(d_ssm, norm_before_gate, group_size = d_ssm / ngroups) (reference
+ * SSD/MedSSD.py:268-269, 393-394).  Rows of `dim` columns, cut into dim / group_size contiguous groups normalised on their own:
+ *   norm_before_gate = 0:  out = rmsnorm_g(x * silu(z)) * w [+ b]
+ *   norm_before_gate = 1:  out = (rmsnorm_g(x) * w [+ b]) * silu(z)
+ *   z == NULL:             out = rmsnorm_g(x) * w [+ b],          rmsnorm_g(v) = v * rsqrt(mean over the group of v^2 + eps)
+ * All arithmetic in fp32.  x, z (rows, dim) in {F32, BF16, F16}, each with its own dtype and row stride in elements, read in place
+ * (z may be a column slice of in_proj's output with any pitch); w (dim) f32; b (dim) f32 or NULL; out (rows, dim) contiguous
+ * out_dtype in {F32, BF16, F16}; rstd (rows, dim / group_size) f32, kept for the backward.
+ * Backward: dy (rows, dim) dy_dtype with row stride dy_row_stride -> dx (rows, dim) x_dtype and dz (rows, dim) z_dtype, contiguous
+ * (dz given exactly when z is); dw_partial, db_partial (b200_rmsnorm_grid(rows, dim, group_size), dim) f32 per-CTA partial sums,
+ * which the caller adds up (no atomics: reproducible); db_partial may be NULL.
+ * group_size must divide dim, dim <= 8192.  Anything else returns < 0 with a message (b200_rmsnorm_grid too).
+ * ------------------------------------------------------------------------------------------ */
+int b200_rmsnorm_grid(int64_t rows, int32_t dim, int32_t group_size);
+int b200_rmsnorm_fwd(const void* x, int32_t x_dtype, int64_t x_row_stride, const void* z, int32_t z_dtype, int64_t z_row_stride,
+                     const float* w, const float* b, void* out, int32_t out_dtype, float* rstd, int64_t rows, int32_t dim,
+                     int32_t group_size, int32_t norm_before_gate, float eps, b200_stream_t stream);
+int b200_rmsnorm_bwd(const void* dy, int32_t dy_dtype, int64_t dy_row_stride, const void* x, int32_t x_dtype, int64_t x_row_stride,
+                     const void* z, int32_t z_dtype, int64_t z_row_stride, const float* w, const float* b, const float* rstd,
+                     void* dx, void* dz, float* dw_partial, float* db_partial, int64_t rows, int32_t dim, int32_t group_size,
+                     int32_t norm_before_gate, b200_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------
  * SS2D output stage (SURVEY.md 8(f) rank 1): out = LayerNorm(y) * silu(z) and its backward -- replaces
  * `y = self.out_norm(y); y = y * F.silu(z)` (reference MedMamba.py:478-479; nn.LayerNorm(d_inner), eps 1e-5)
  * and the four autograd kernels behind it.

@@ -99,6 +99,9 @@ SIGNATURES = {
     "b200_ssd_bwd": (C.c_int, [C.POINTER(SsdBwdParams), vp]),
     "b200_rmsnorm_gated_fwd": (C.c_int, [vp, vp, vp, vp, vp, i64, i32, f32, vp]),
     "b200_rmsnorm_gated_bwd": (C.c_int, [vp, vp, vp, vp, vp, vp, vp, vp, i32, i64, i32, vp]),
+    "b200_rmsnorm_grid": (C.c_int, [i64, i32, i32]),
+    "b200_rmsnorm_fwd": (C.c_int, [vp, i32, i64, vp, i32, i64, vp, vp, vp, i32, vp, i64, i32, i32, i32, f32, vp]),
+    "b200_rmsnorm_bwd": (C.c_int, [vp, i32, i64, vp, i32, i64, vp, i32, i64, vp, vp, vp, vp, vp, vp, vp, i64, i32, i32, i32, vp]),
     "b200_ln_gate_grid": (C.c_int, [i64]),
     "b200_ln_gate_fwd": (C.c_int, [vp, i32, i64, vp, i64, i32, vp, vp, vp, i32, vp, vp, i64, i32, f32, vp]),
     "b200_ln_gate_bwd": (C.c_int, [vp, vp, i32, i64, vp, i64, i32, vp, vp, i32, vp, vp, vp, vp, vp, vp, i64, i32, vp]),
@@ -187,6 +190,15 @@ def is_dense(t) -> bool:
             return False
         expect *= size
     return True
+
+
+def rows_view(t, D):
+    """(tensor, row stride) such that row r of the flattened (..., D) tensor starts at data_ptr + r * stride elements;
+    views whose leading dimensions collapse (e.g. one half of a chunk(2, -1)) are used in place."""
+    if t.is_contiguous():
+        return t, D
+    ok = t.dim() >= 2 and t.stride(-1) == 1 and all(t.stride(i) == t.stride(i + 1) * t.shape[i + 1] for i in range(t.dim() - 2))
+    return (t, t.stride(-2)) if ok else (t.contiguous(), D)
 
 
 def no_autocast(fn):

@@ -26,15 +26,6 @@ from .cross import ss2d_core
 from .selective_scan_interface import selective_scan_fn
 
 
-def _rows_view(t, D):
-    """(tensor, row stride) such that row r of the flattened (..., D) tensor starts at data_ptr + r * stride elements;
-    views whose leading dimensions collapse (e.g. one half of a chunk(2, -1)) are used in place."""
-    if t.is_contiguous():
-        return t, D
-    ok = t.dim() >= 2 and t.stride(-1) == 1 and all(t.stride(i) == t.stride(i + 1) * t.shape[i + 1] for i in range(t.dim() - 2))
-    return (t, t.stride(-2)) if ok else (t.contiguous(), D)
-
-
 class SplitHalvesFn(torch.autograd.Function):
     """a, b = t.chunk(2, dim=-1) (MedMamba.py:467 `x, z = xz.chunk(2, dim=-1)`, :530 `left, right = input.chunk(...)`) with a
     one-pass backward: d(input) = cat(d left, d right)
@@ -72,12 +63,12 @@ class LnGateFn(torch.autograd.Function):
         D = y.shape[-1]
         if y.dtype != torch.float32 and not (y.dtype == torch.bfloat16 and z is None):
             y = y.float()
-        y2, ys = _rows_view(y, D)
+        y2, ys = _lib.rows_view(y, D)
         z2, zs = (None, 0)
         if z is not None:
             if z.dtype not in (torch.float32, torch.bfloat16):
                 z = z.float()
-            z2, zs = _rows_view(z, D)
+            z2, zs = _lib.rows_view(z, D)
         rows = y.numel() // D
         w32, b32 = weight.detach().float().contiguous(), bias.detach().float().contiguous()
         out = torch.empty((rows, D), dtype=out_dtype, device=y.device)

@@ -7,8 +7,9 @@ norm.weight, out_proj.weight`), so reference checkpoints load with strict=True, 
 
 The scan itself is `mamba_chunk_scan_combined` from .ssd_combined (libb200ssm, csrc/ssd.cu), called
 with exactly the tensors the reference builds (SSD/MedSSD.py:332-375): (b, l, .) views of
-channel-major storage, one group of 4*d_state states shared by all 4*nheads heads.  The gated RMSNorm
-(`mamba_ssm...layernorm_gated.RMSNorm`, SSD/MedSSD.py:268-269,393-394) is .ssd_combined.RMSNormGated.
+channel-major storage, ngroups groups of 4*d_state states (one in the reference).  The gated RMSNorm
+(`mamba_ssm...layernorm_gated.RMSNorm`, SSD/MedSSD.py:268-269,393-394) is .ssd_combined.RMSNormGated, with
+group_size = d_ssm / ngroups and either order of norm and gate.
 Tensor / sequence parallel branches of the reference constructor (process_group is always None
 there, SURVEY.md 2.4) are not mirrored.
 """
@@ -22,7 +23,7 @@ import torch.nn.functional as F
 
 from . import _lib
 from .cross import cross_scan4_split, ssd_merge4
-from .ss2d import DwConvSiluFn
+from .ss2d import DwConvSiluFn, _autocast_out_dtype
 from .ssd_combined import RMSNormGated, mamba_chunk_scan_combined
 
 
@@ -107,7 +108,7 @@ class SS2D_with_SSD(nn.Module):
         out = ssd_merge4(y, H, W).view(B, H, W, -1)                                             # one gather pass (csrc/cross.cu)
 
         if self.rmsnorm:
-            out = self.norm(out, z)
+            out = self.norm(out, z, out_dtype=_autocast_out_dtype())   # z read in place from zxbcdt; bf16 out under bf16 autocast
         if d_mlp > 0:
             out = torch.cat([F.silu(z0) * x0, out], dim=-1)
         out = self.out_proj(out.to(self.out_proj.weight.dtype) if not torch.is_autocast_enabled() else out)

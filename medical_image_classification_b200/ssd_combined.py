@@ -210,62 +210,98 @@ def mamba_chunk_scan_combined(x, dt, A, B, C, chunk_size, D=None, z=None, dt_bia
 
 
 # ------------------------------------------------------------------------------------------------
-# gated RMSNorm (mamba_ssm.ops.triton.layernorm_gated.RMSNorm as used at SSD/MedSSD.py:268-269,393-394)
+# gated RMSNorm (mamba_ssm.ops.triton.layernorm_gated.RMSNorm / rmsnorm_fn, mamba_ssm 2.2.2, as used at
+# SSD/MedSSD.py:268-269,393-394): csrc/rmsnorm.cu through b200_rmsnorm_fwd / _bwd
 # ------------------------------------------------------------------------------------------------
+_IO_DTYPES = (torch.float32, torch.bfloat16, torch.float16)
+
+
+def _rows_io(t, dim):
+    """(tensor, row stride) of t as the kernels read it: in place when its dtype is one they read and its rows are contiguous."""
+    return _lib.rows_view(t if t.dtype in _IO_DTYPES else t.float(), dim)
+
+
 class RmsNormGatedFn(torch.autograd.Function):
-    """y = rmsnorm(x * silu(z)) * w over the last dimension (norm_before_gate=False, one group)."""
+    """out = rmsnorm_g(x * silu(z)) * w + b (norm_before_gate=False), (rmsnorm_g(x) * w + b) * silu(z) (True), or
+    rmsnorm_g(x) * w + b (z None), each group of group_size columns normalised on its own.  x, z and dy are read in place when
+    their rows are contiguous (z is a column slice of in_proj's output); out is out_dtype; gradients come back in the primals'
+    dtypes."""
 
     @staticmethod
     @_no_autocast
-    def forward(ctx, x, z, w, eps):
-        _lib.require_cuda(x, z, w)
-        shape = x.shape
-        dim = shape[-1]
-        x2 = x.reshape(-1, dim).float().contiguous()
-        z2 = z.reshape(-1, dim).float().contiguous()
-        w32 = w.float().contiguous()
-        rows = x2.shape[0]
-        y = torch.empty_like(x2)
-        rstd = torch.empty(rows, dtype=torch.float32, device=x.device)
-        _lib.launch("b200_rmsnorm_gated_fwd", x.device, x2.data_ptr(), z2.data_ptr(), w32.data_ptr(), y.data_ptr(), rstd.data_ptr(),
-                    rows, dim, float(eps))
-        ctx.save_for_backward(x2, z2, w32, rstd)
-        ctx.meta = (shape, x.dtype, z.dtype, w.dtype)
-        return y.view(shape).to(x.dtype)
+    def forward(ctx, x, z, weight, bias, eps, group_size, norm_before_gate, out_dtype):
+        _lib.require_cuda(x, z, weight, bias)
+        dim = x.shape[-1]
+        rows = x.numel() // dim
+        x2, xs = _rows_io(x, dim)
+        z2, zs = _rows_io(z, dim) if z is not None else (None, 0)
+        w32, b32 = _lib.f32c(weight), _lib.f32c(bias)
+        out = torch.empty((rows, dim), dtype=out_dtype, device=x.device)
+        rstd = torch.empty((rows, dim // group_size), dtype=torch.float32, device=x.device)
+        _lib.launch("b200_rmsnorm_fwd", x.device, x2.data_ptr(), _lib.dtype_code(x2.dtype), xs, _lib.ptr(z2),
+                    _lib.dtype_code(z2.dtype) if z2 is not None else 0, zs, w32.data_ptr(), _lib.ptr(b32), out.data_ptr(),
+                    _lib.dtype_code(out_dtype), rstd.data_ptr(), rows, dim, group_size, int(norm_before_gate), float(eps))
+        ctx.save_for_backward(x2, z2, w32, b32, rstd)
+        ctx.cfg = (xs, zs, rows, group_size, int(norm_before_gate))
+        ctx.dtypes = (x.dtype, None if z is None else z.dtype, weight.dtype, None if bias is None else bias.dtype)
+        return out.view(x.shape)
 
     @staticmethod
     @_no_autocast
     def backward(ctx, dy):
-        x2, z2, w32, rstd = ctx.saved_tensors
-        shape, xdt, zdt, wdt = ctx.meta
-        rows, dim = x2.shape
-        dy2 = dy.reshape(-1, dim).float().contiguous()
-        dx = torch.empty_like(x2)
-        dz = torch.empty_like(x2)
-        nblk = int(min(rows, 592))
-        dwp = torch.empty((nblk, dim), dtype=torch.float32, device=x2.device)
-        _lib.launch("b200_rmsnorm_gated_bwd", x2.device, x2.data_ptr(), z2.data_ptr(), w32.data_ptr(), rstd.data_ptr(), dy2.data_ptr(),
-                    dx.data_ptr(), dz.data_ptr(), dwp.data_ptr(), nblk, rows, dim)
-        return dx.view(shape).to(xdt), dz.view(shape).to(zdt), dwp.sum(0).to(wdt), None
+        x2, z2, w32, b32, rstd = ctx.saved_tensors
+        xs, zs, rows, group_size, nbg = ctx.cfg
+        t_x, t_z, t_w, t_b = ctx.dtypes
+        shape, dim, dev = dy.shape, dy.shape[-1], dy.device
+        dy2, dys = _rows_io(dy, dim)
+        dx = torch.empty((rows, dim), dtype=x2.dtype, device=dev)
+        dz = torch.empty((rows, dim), dtype=z2.dtype, device=dev) if z2 is not None else None
+        grid = _lib.load().b200_rmsnorm_grid(rows, dim, group_size)
+        if grid < 0:
+            _lib.check(grid, "b200_rmsnorm_grid")
+        part = torch.empty((1 if b32 is None else 2, grid, dim), dtype=torch.float32, device=dev)
+        _lib.launch("b200_rmsnorm_bwd", dev, dy2.data_ptr(), _lib.dtype_code(dy2.dtype), dys, x2.data_ptr(), _lib.dtype_code(x2.dtype),
+                    xs, _lib.ptr(z2), _lib.dtype_code(z2.dtype) if z2 is not None else 0, zs, w32.data_ptr(), _lib.ptr(b32),
+                    rstd.data_ptr(), dx.data_ptr(), _lib.ptr(dz), part[0].data_ptr(), part[1].data_ptr() if b32 is not None else None,
+                    rows, dim, group_size, nbg)
+        dwb = part.sum(1)
+        return (dx.view(shape).to(t_x), None if dz is None else dz.view(shape).to(t_z), dwb[0].to(t_w),
+                None if b32 is None else dwb[1].to(t_b), None, None, None, None)
+
+
+def _rmsnorm(x, z, weight, bias, eps, group_size, norm_before_gate, out_dtype):
+    dim = x.shape[-1]
+    group_size = dim if group_size is None else int(group_size)
+    if z is not None and z.shape != x.shape:
+        raise RuntimeError(f"rmsnorm: z {tuple(z.shape)} must have the shape of x {tuple(x.shape)}")
+    if tuple(weight.shape) != (dim,) or (bias is not None and tuple(bias.shape) != (dim,)):
+        raise RuntimeError(f"rmsnorm: weight / bias must be ({dim},)")
+    if group_size < 1 or dim % group_size:
+        raise RuntimeError(f"rmsnorm: group_size {group_size} does not divide the last dimension {dim}")
+    return RmsNormGatedFn.apply(x, z, weight, bias, eps, group_size, bool(norm_before_gate), out_dtype)
+
+
+def rmsnorm_fn(x, weight, bias, z=None, eps=1e-6, group_size=None, norm_before_gate=True):
+    """mamba_ssm.ops.triton.layernorm_gated.rmsnorm_fn (mamba_ssm 2.2.2): the gated, grouped RMSNorm of rms_norm_ref; out in
+    x's dtype."""
+    return _rmsnorm(x, z, weight, bias, eps, group_size, norm_before_gate, x.dtype)
 
 
 class RMSNormGated(torch.nn.Module):
-    """Mirror of mamba_ssm's gated RMSNorm module for the configuration the reference uses
-    (norm_before_gate=False, group_size == hidden_size): y = rmsnorm(x * silu(z)) * weight."""
+    """Mirror of mamba_ssm's gated RMSNorm module (layernorm_gated.RMSNorm): rmsnorm_fn with this module's weight, group_size
+    (None: one group of hidden_size) and norm_before_gate; z may be None."""
 
     def __init__(self, hidden_size, eps=1e-5, group_size=None, norm_before_gate=False, device=None, dtype=None):
         super().__init__()
-        if norm_before_gate:
-            raise NotImplementedError("RMSNormGated: norm_before_gate=True is not used by the reference models")
-        if group_size is not None and group_size != hidden_size:
-            raise NotImplementedError("RMSNormGated: only one normalisation group (group_size == hidden_size)")
+        if group_size is not None and (group_size < 1 or hidden_size % group_size):
+            raise ValueError(f"RMSNormGated: group_size {group_size} does not divide hidden_size {hidden_size}")
         self.eps = eps
         self.weight = torch.nn.Parameter(torch.ones(hidden_size, device=device, dtype=dtype))
         self.register_parameter("bias", None)
         self.group_size = group_size
         self.norm_before_gate = norm_before_gate
 
-    def forward(self, x, z=None):
-        if z is None:
-            raise NotImplementedError("RMSNormGated: the reference always passes the gate z (SSD/MedSSD.py:394)")
-        return RmsNormGatedFn.apply(x, z, self.weight, self.eps)
+    def forward(self, x, z=None, out_dtype=None):
+        """out_dtype (default x.dtype, mamba_ssm's contract) lets a caller ask for what its next Linear casts to under autocast."""
+        return _rmsnorm(x, z, self.weight, self.bias, self.eps, self.group_size, self.norm_before_gate,
+                        x.dtype if out_dtype is None else out_dtype)
