@@ -203,10 +203,20 @@ int b200_ssd_merge4_bwd(const float* dout, float* dy, int32_t batch, int32_t d, 
  *
  * x, out (batch, L, H, P); dt (batch, L, H); B, C (batch, L, G, N); A, D, dt_bias (H) f32.
  * Every tensor is addressed by explicit element strides (the reference passes permuted views
- * whose L stride is 1, SURVEY.md section 3.3).  The gate z, D with a head dimension, seq_idx and
- * cu_seqlens are never passed by the reference models (SSD/MedSSD.py:361-375) and are rejected
+ * whose L stride is 1, SURVEY.md section 3.3).  The gate z and D with a head dimension are applied
  * by the host wrapper.  Evaluated chunk-wise (chunk_size steps): Y = (C B^T o decay) (dt X) +
  * decay C S_prev, S_c = decay S_{c-1} + B^T (decay dt X); all contractions on tensor cores.
+ *
+ * Packed variable-length rows (mamba_ssm 2.2.2's seq_idx): seq_idx (batch, L) int32, non-decreasing
+ * along L (not checked).  The recurrence restarts wherever seq_idx changes: S_t = dt'_t x_t B_t when
+ * seq_idx[t] != seq_idx[t-1], and initial_states reach only positions whose id equals 0 before the
+ * first change.  final_states is the state after the row's last token.  The backward applies the
+ * same masks.  seq_idx == NULL is a row of one sequence.
+ *
+ * b200_ssd_varlen_states (batch == 1): after b200_ssd_fwd on the same params and workspace, writes
+ * states (nseq, H, P, N) f32 contiguous, the state after the last token of each sequence
+ * [cu_seqlens[k], cu_seqlens[k+1]) (values clamped into [0, seqlen]; an empty sequence gets zeros).
+ * The first sequence (starting at 0) includes initial_states.
  * ------------------------------------------------------------------------------------------ */
 typedef struct {
     int32_t batch, seqlen, nheads, headdim, n_groups, dstate, chunk_size;
@@ -233,6 +243,8 @@ typedef struct {
     float* workspace;      /* b200_ssd_workspace_bytes() bytes, kept for the backward:
                               dt' [b][h][c][Q] | cumsum(dt' A) [b][h][c][Q] | chunk-entry states
                               [b][c][h][P][N] | C B^T [b][c][g][Q][Q] */
+    const int32_t* seq_idx;      /* (batch, L) int32 or NULL */
+    int64_t seq_idx_stride[2];   /* batch, L; non-negative */
 } b200_ssd_fwd_params;
 
 typedef struct {
@@ -264,6 +276,8 @@ size_t b200_ssd_bwd_scratch_bytes(int32_t batch, int32_t seqlen, int32_t nheads,
                                   int32_t n_groups, int32_t dstate, int32_t chunk_size);
 int b200_ssd_fwd(const b200_ssd_fwd_params* p, b200_stream_t stream);
 int b200_ssd_bwd(const b200_ssd_bwd_params* p, b200_stream_t stream);
+int b200_ssd_varlen_states(const b200_ssd_fwd_params* p, const int32_t* cu_seqlens, int32_t nseq, float* states,
+                           b200_stream_t stream);
 
 /* Gated RMSNorm used by SS2D_with_SSD (reference SSD/MedSSD.py:268-269,393-394;
  * mamba_ssm.ops.triton.layernorm_gated.RMSNorm with norm_before_gate=False, one group):

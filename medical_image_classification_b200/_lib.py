@@ -58,6 +58,7 @@ class SsdFwdParams(C.Structure):
         ("out_stride", i64 * 4),
         ("x", vp), ("dt", vp), ("A", vp), ("B", vp), ("C", vp), ("D", vp), ("dt_bias", vp),
         ("initial_states", vp), ("out", vp), ("final_states", vp), ("workspace", vp),
+        ("seq_idx", vp), ("seq_idx_stride", i64 * 2),
     ]
 
 
@@ -97,6 +98,7 @@ SIGNATURES = {
     "b200_ssd_bwd_scratch_bytes": (C.c_size_t, [i32] * 7),
     "b200_ssd_fwd": (C.c_int, [C.POINTER(SsdFwdParams), vp]),
     "b200_ssd_bwd": (C.c_int, [C.POINTER(SsdBwdParams), vp]),
+    "b200_ssd_varlen_states": (C.c_int, [C.POINTER(SsdFwdParams), vp, i32, vp, vp]),
     "b200_rmsnorm_gated_fwd": (C.c_int, [vp, vp, vp, vp, vp, i64, i32, f32, vp]),
     "b200_rmsnorm_gated_bwd": (C.c_int, [vp, vp, vp, vp, vp, vp, vp, vp, i32, i64, i32, vp]),
     "b200_rmsnorm_grid": (C.c_int, [i64, i32, i32]),

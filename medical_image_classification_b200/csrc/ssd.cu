@@ -34,9 +34,29 @@ constexpr int A_FLOATS = (BK * LDA_KM > BM * LDA_MK) ? BK * LDA_KM : BM * LDA_MK
 constexpr int B_FLOATS = (BK * LDB_KN > BN * LDB_NK) ? BK * LDB_KN : BN * LDB_NK;  // 2304
 constexpr int MAXQ = 256;
 
+// seq_idx (batch, L): packed variable-length rows; p == NULL is one sequence per row
+struct Seq {
+    const int32_t* p;
+    int64_t s0, s1;
+    __device__ __forceinline__ int at(int b, int l) const { return __ldg(p + b * s0 + (int64_t)l * s1); }
+};
+
 struct Dims {
     int batch, L, H, P, G, N, Q, nc, hpg;
+    Seq seq;
 };
+
+// Masks of a packed row (seq_idx non-decreasing): with sid(l) = seq_idx[b][l], for chunk c of row b
+//   intra-chunk term (l, s):       sid(l) == sid(s)
+//   chunk-entry term at l:         sid(l) == seq_prev(c)   (the id at the previous chunk's last position, 0 before chunk 0)
+//   chunk-state contribution of s: sid(s) == seq_end(c)    (the id at this chunk's last position)
+//   state passing into chunk c+1:  seq_end(c) == seq_prev(c)
+// The backward applies the same masks to the adjoint.  Each is a per-row or per-column factor of a contraction except the
+// intra-chunk one, which the SEQ instantiations apply per element where the causal mask already is.
+__device__ __forceinline__ int seq_prev(const Dims& d, int b, int c) { return c > 0 ? d.seq.at(b, c * d.Q - 1) : 0; }
+__device__ __forceinline__ int seq_end(const Dims& d, int b, int c) { return d.seq.at(b, min((c + 1) * d.Q, d.L) - 1); }
+// seq_idx of chunk c's position i (positions past the end of the row repeat the last id)
+__device__ __forceinline__ int seq_at(const Dims& d, int b, int c, int i) { return d.seq.at(b, min(c * d.Q + i, d.L - 1)); }
 
 struct Ws {  // views into the forward workspace
     float* dtp;     // [b][h][nc][Q]
@@ -54,6 +74,7 @@ static Dims make_dims(const b200_ssd_fwd_params& p) {
     d.batch = p.batch; d.L = p.seqlen; d.H = p.nheads; d.P = p.headdim; d.G = p.n_groups; d.N = p.dstate; d.Q = p.chunk_size;
     d.nc = (p.seqlen + p.chunk_size - 1) / p.chunk_size;
     d.hpg = p.nheads / p.n_groups;
+    d.seq = Seq{p.seq_idx, p.seq_idx_stride[0], p.seq_idx_stride[1]};
     return d;
 }
 static Ws make_ws(float* base, const Dims& d) {
@@ -287,6 +308,7 @@ struct Smem {
     float v2[2][MAXQ];
     float rowf[MAXQ / BK][BM];    // per (k-tile, row) decay factors of the diagonal-block contractions
     float red[8];
+    int sid[MAXQ];                // seq_idx of the chunk's positions (SEQ instantiations)
 };
 
 // One software-pipelined pass over nkt k-tiles: the raw tile kt+1 is fetched into registers while the
@@ -365,6 +387,7 @@ struct Shared {
     float v2[2][MAXQ];
     float rowf[MAXQ / BK][BM];
     float red[8];
+    int sid[MAXQ];
     uint64_t bar[2];      // "the MMAs that read operand stage s have completed"
     uint64_t bar_done;
     uint32_t tmem_slot, pad_;
@@ -634,6 +657,12 @@ __device__ __forceinline__ void stage_cs(S& sm, int hb, const Ws& ws, const Dims
     }
 }
 
+// stage chunk c's seq_idx values into shared memory (no barrier)
+template <class S>
+__device__ __forceinline__ void stage_sid(S& sm, const Dims& d, int b, int c) {
+    for (int i = threadIdx.x; i < d.Q; i += NTHR) sm.sid[i] = seq_at(d, b, c, i);
+}
+
 template <class S>
 __device__ __forceinline__ float block_sum(S& sm, float v) {
 #pragma unroll
@@ -684,7 +713,7 @@ __global__ void __launch_bounds__(MAXQ) dt_cumsum_kernel(const T* dt, int64_t s0
 //   MODE 0 (chunk states):  src_x = x,    src_b = B,  w_s = exp(cs_Q - cs_s) dt'_s
 //   MODE 1 (d states):      src_x = dout, src_b = C,  w_s = exp(cs_s)
 // GEMM: M = n (128 per tile), N = p (64 per tile), K = s.
-template <typename T, int MODE, class E>
+template <typename T, int MODE, class E, bool SEQ>
 __global__ void __launch_bounds__(NTHR, E::MIN_CTAS) chunk_state_kernel(View4<T> X, View4<T> Bv, Dims d, Ws ws, float* out, int x3) {
     typename E::Shared& sm = E::smem();
     const int ntn = (d.N + BM - 1) / BM, ntp = (d.P + BN - 1) / BN;
@@ -702,6 +731,11 @@ __global__ void __launch_bounds__(NTHR, E::MIN_CTAS) chunk_state_kernel(View4<T>
     const float csQ = sm.cs[0][d.Q - 1];
     for (int i = threadIdx.x; i < d.Q; i += NTHR)
         sm.v1[0][i] = MODE == 0 ? exp_acc(csQ - sm.cs[0][i]) * sm.dtp[0][i] : exp_acc(sm.cs[0][i]);
+    if (SEQ) {   // MODE 0: only the sequence still open at the chunk's end; MODE 1: only the one entering the chunk
+        const int ref = MODE == 0 ? seq_end(d, b, c) : seq_prev(d, b, c);
+        for (int i = threadIdx.x; i < d.Q; i += NTHR)
+            if (seq_at(d, b, c, i) != ref) sm.v1[0][i] = 0.f;
+    }
     __syncthreads();
     const T* pa = Bv.p + b * Bv.s0 + (int64_t)l0 * Bv.s1 + g * Bv.s2 + (int64_t)n0 * Bv.s3;   // (i = n, k = s)
     const T* pb = X.p + b * X.s0 + (int64_t)l0 * X.s1 + h * X.s2 + (int64_t)p0 * X.s3;        // (i = p, k = s)
@@ -729,6 +763,7 @@ __global__ void __launch_bounds__(NTHR, E::MIN_CTAS) chunk_state_kernel(View4<T>
 // HBM-bound streaming pass: 128-bit accesses, 32-bit indexing, and the loads of 8 chunks are issued before the
 // (sequential) recurrence over them so each thread keeps 8 independent 16-byte requests in flight.
 constexpr int SPB = 8;  // chunks per batch of loads
+template <bool SEQ>
 __global__ void __launch_bounds__(256) state_pass_kernel(Dims d, Ws ws, const float* init, float* fin) {
     const int PN4 = d.P * d.N / 4;
     const int e = blockIdx.x * blockDim.x + threadIdx.x;
@@ -746,6 +781,7 @@ __global__ void __launch_bounds__(256) state_pass_kernel(Dims d, Ws ws, const fl
             if (c0 + k < d.nc) {
                 loc[k] = st[(size_t)(c0 + k) * cstride];
                 dec[k] = exp_acc(__ldg(csq + (size_t)(c0 + k) * d.Q));
+                if (SEQ && seq_end(d, b, c0 + k) != seq_prev(d, b, c0 + k)) dec[k] = 0.f;   // a sequence starts in the chunk
             }
 #pragma unroll
         for (int k = 0; k < SPB; ++k)
@@ -758,6 +794,7 @@ __global__ void __launch_bounds__(256) state_pass_kernel(Dims d, Ws ws, const fl
     if (fin) reinterpret_cast<float4*>(fin)[((size_t)b * d.H + h) * PN4 + e] = run;
 }
 // element-wise fallback (P * N not a multiple of 4)
+template <bool SEQ>
 __global__ void state_pass_kernel_scalar(Dims d, Ws ws, const float* init, float* fin) {
     const size_t PN = (size_t)d.P * d.N;
     const size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -770,7 +807,8 @@ __global__ void state_pass_kernel_scalar(Dims d, Ws ws, const float* init, float
         const float loc = *s;
         *s = run;
         const float csQ = ws.cs[(((size_t)b * d.H + h) * d.nc + c) * d.Q + d.Q - 1];
-        run = exp_acc(csQ) * run + loc;
+        const float dec = (SEQ && seq_end(d, b, c) != seq_prev(d, b, c)) ? 0.f : exp_acc(csQ);
+        run = dec * run + loc;
     }
     if (fin) fin[idx] = run;
 }
@@ -813,7 +851,7 @@ __global__ void __launch_bounds__(NTHR, E::MIN_CTAS) cb_kernel(View4<T> Cv, View
 // 32-wide k-tile it is the product of two factors <= 1 (reference point: cs at the end of the k-tile), one
 // per row and one per column, precomputed once per CTA; inside the 32 x 32 diagonal block it is evaluated
 // exactly per element (no overflow whatever the decay rate).
-template <typename T, class E>
+template <typename T, class E, bool SEQ>
 __global__ void __launch_bounds__(NTHR, E::MIN_CTAS) chunk_scan_kernel(View4<T> X, View4<T> Cv, const float* D, Dims d, Ws ws, T* out,
                                                              int64_t o0, int64_t o1, int64_t o2, int64_t o3, int has_init, int x3) {
     typename E::Shared& sm = E::smem();
@@ -829,12 +867,15 @@ __global__ void __launch_bounds__(NTHR, E::MIN_CTAS) chunk_scan_kernel(View4<T> 
     const int m0 = tm * BM, p0 = tp * BN;
     if (m0 >= q) return;
     stage_cs(sm, 0, ws, d, b, h, c);
+    if (SEQ) stage_sid(sm, d, b, c);
     __syncthreads();
     const int send = min(q, m0 + BM), nkt1 = (send + BK - 1) / BK;
+    const int sprev = SEQ ? seq_prev(d, b, c) : 0;
     for (int i = threadIdx.x; i < d.Q; i += NTHR) {
         const float ref = sm.cs[0][min((i / BK) * BK + BK - 1, d.Q - 1)];
         sm.v1[0][i] = exp_acc(ref - sm.cs[0][i]) * sm.dtp[0][i];   // column factor (<= dt')
         sm.v2[0][i] = exp_acc(sm.cs[0][i]);                        // exp(cs_l) of the state term
+        if (SEQ && sm.sid[i] != sprev) sm.v2[0][i] = 0.f;          // the chunk-entry state belongs to another sequence
     }
     for (int idx = threadIdx.x; idx < nkt1 * BM; idx += NTHR) {
         const int kt = idx / BM, i = idx % BM;
@@ -856,6 +897,7 @@ __global__ void __launch_bounds__(NTHR, E::MIN_CTAS) chunk_scan_kernel(View4<T> 
             E::template store<BM, false>(sA, r, [&](int i, int k, float v) {
                 const int l = m0 + i, s = k0 + k;
                 if (s > l) return 0.f;
+                if (SEQ && sm.sid[min(l, d.Q - 1)] != sm.sid[s]) return 0.f;
                 if (l < k0 + BK) return v * exp_acc(sm.cs[0][l] - sm.cs[0][s]) * sm.dtp[0][s];
                 return v * sm.rowf[kt][i] * sm.v1[0][s];
             });
@@ -889,6 +931,7 @@ __global__ void __launch_bounds__(NTHR, E::MIN_CTAS) chunk_scan_kernel(View4<T> 
 //          dcsQ[b][h][c] = <G[c], Sin[c+1]>  (accumulated with atomics; caller zero-fills) ----------
 // Same streaming structure as K3 (128-bit, 8 chunks of loads in flight); the per-chunk dot products are kept in
 // registers and block-reduced once per batch of chunks.
+template <bool SEQ>
 __global__ void __launch_bounds__(NTHR) state_pass_bwd_kernel(Dims d, Ws ws, float* dstates, float* dcsQ) {
     __shared__ float red[NTHR / 32][SPB];
     const int PN4 = d.P * d.N / 4;
@@ -913,6 +956,7 @@ __global__ void __launch_bounds__(NTHR) state_pass_bwd_kernel(Dims d, Ws ws, flo
                 if (ok) off[k] = ds[(size_t)c * cstride];
                 if (ok && c + 1 < d.nc) nxt[k] = sn[(size_t)(c + 1) * cstride];
                 dec[k] = exp_acc(__ldg(csq + (size_t)c * d.Q));
+                if (SEQ && seq_end(d, b, c) != seq_prev(d, b, c)) dec[k] = 0.f;   // no adjoint carry across a reset
             }
         }
 #pragma unroll
@@ -946,6 +990,7 @@ __global__ void __launch_bounds__(NTHR) state_pass_bwd_kernel(Dims d, Ws ws, flo
     }
 }
 // element-wise fallback (P * N not a multiple of 4)
+template <bool SEQ>
 __global__ void __launch_bounds__(NTHR) state_pass_bwd_kernel_scalar(Dims d, Ws ws, float* dstates, float* dcsQ) {
     __shared__ float red[NTHR / 32];
     const size_t PN = (size_t)d.P * d.N;
@@ -975,13 +1020,14 @@ __global__ void __launch_bounds__(NTHR) state_pass_bwd_kernel_scalar(Dims d, Ws 
         }
         __syncthreads();
         const float csQ = ws.cs[(((size_t)b * d.H + h) * d.nc + c) * d.Q + d.Q - 1];
-        run = off + exp_acc(csQ) * run;
+        const float dec = (SEQ && seq_end(d, b, c) != seq_prev(d, b, c)) ? 0.f : exp_acc(csQ);
+        run = off + dec * run;
     }
 }
 
 // ---- B3: Z = (CB o decay)^T dout + exp(cs_Q - cs) B G^T;  dx = dt' Z + D dout;
 //          ddtp_exp[s] = sum_p x Z;  dcs_pos[l] = sum_p dout (out - D x);  dD += sum dout x --------
-template <typename T>
+template <typename T, bool SEQ>
 __global__ void __launch_bounds__(NTHR, 2) dx_kernel(View4<T> X, View4<T> Bv, View4<T> DO, View4<T> OUT, const float* D, Dims d, Ws ws,
                                                      const float* G, float* dx, OutS dxs, float* ddtp_exp, float* dcs_pos, float* dD, int x3) {
     Smem& sm = smem_ref();
@@ -997,8 +1043,10 @@ __global__ void __launch_bounds__(NTHR, 2) dx_kernel(View4<T> X, View4<T> Bv, Vi
     const int m0 = tm * BM, p0 = tp * BN;
     if (m0 >= q) return;
     stage_cs(sm, 0, ws, d, b, h, c);
+    if (SEQ) stage_sid(sm, d, b, c);
     __syncthreads();
     const float csQ = sm.cs[0][d.Q - 1];
+    const int send_id = SEQ ? seq_end(d, b, c) : 0;
     const float* cb = ws.cb + (((size_t)b * d.nc + c) * d.G + g) * (size_t)d.Q * d.Q;
     const float* Gs = G + (((size_t)b * d.nc + c) * d.H + h) * (size_t)d.P * d.N;
     const bool do_ifast = DO.s3 < DO.s1, b_ifast = Bv.s1 <= Bv.s3;
@@ -1008,6 +1056,7 @@ __global__ void __launch_bounds__(NTHR, 2) dx_kernel(View4<T> X, View4<T> Bv, Vi
     for (int k0 = (m0 / BK) * BK; k0 < q; k0 += BK, buf ^= 1) {  // l >= s
         fill_tile<BM, true>(sm.A[buf], true, [&](int i, int k) {
             const int s = m0 + i, l = k0 + k;
+            if (SEQ && l < q && s <= l && sm.sid[l] != sm.sid[s]) return 0.f;
             return (l < q && s <= l) ? cb[(size_t)l * d.Q + s] * exp_acc(sm.cs[0][l] - sm.cs[0][s]) : 0.f;
         });
         fill_tile<BN, false>(sm.B[buf], do_ifast, [&](int i, int k) {
@@ -1021,6 +1070,7 @@ __global__ void __launch_bounds__(NTHR, 2) dx_kernel(View4<T> X, View4<T> Bv, Vi
         for (int k0 = 0; k0 < d.N; k0 += BK, buf ^= 1) {
             fill_tile<BM, true>(sm.A[buf], b_ifast, [&](int i, int k) {
                 const int s = m0 + i, n = k0 + k;
+                if (SEQ && s < q && sm.sid[s] != send_id) return 0.f;
                 return (s < q && n < d.N) ? Bv.at(b, l0 + s, g, n) * exp_acc(csQ - sm.cs[0][s]) : 0.f;
             });
             fill_tile<BN, false>(sm.B[buf], false, [&](int i, int k) {
@@ -1076,7 +1126,7 @@ __global__ void __launch_bounds__(NTHR, 2) dx_kernel(View4<T> X, View4<T> Bv, Vi
 
 // B3 on the tcgen05 engine: same contractions, operands staged through registers (128-bit loads where the view
 // allows) into UMMA tiles, accumulator row = one thread in the epilogue (row sums need no shuffles).
-template <typename T>
+template <typename T, bool SEQ>
 __global__ void __launch_bounds__(NTHR, TcEngine::MIN_CTAS) dx_kernel_tc(View4<T> X, View4<T> Bv, View4<T> DO, View4<T> OUT, const float* D, Dims d, Ws ws,
                                                         const float* G, float* dx, OutS dxs, float* ddtp_exp, float* dcs_pos, float* dD, int x3) {
     using E = TcEngine;
@@ -1093,6 +1143,7 @@ __global__ void __launch_bounds__(NTHR, TcEngine::MIN_CTAS) dx_kernel_tc(View4<T
     const int m0 = tm * BM, p0 = tp * BN;
     if (m0 >= q) return;
     stage_cs(sm, 0, ws, d, b, h, c);
+    if (SEQ) stage_sid(sm, d, b, c);
     __syncthreads();
     const float csQ = sm.cs[0][d.Q - 1];
     const float* cb = ws.cb + (((size_t)b * d.nc + c) * d.G + g) * (size_t)d.Q * d.Q;
@@ -1111,13 +1162,18 @@ __global__ void __launch_bounds__(NTHR, TcEngine::MIN_CTAS) dx_kernel_tc(View4<T
                 const int k0 = kb + kt * BK;
                 E::template store_any<BM>(dst, r, true, [&](int i, int k, float v) {
                     const int sidx = m0 + i, l = k0 + k;
+                    if (SEQ && l < q && sidx <= l && sm.sid[l] != sm.sid[sidx]) return 0.f;
                     return (l < q && sidx <= l) ? v * exp_acc(sm.cs[0][l] - sm.cs[0][sidx]) : 0.f;
                 });
             },
             [&](int, const RegTile<BN>& r, const tc::Dst& dst) { E::template store_any<BN>(dst, r, kib, Identity()); });
     }
     if (c + 1 < d.nc) {   // Z += exp(cs_Q - cs_s) B G^T (G of the last chunk is identically zero)
-        if (threadIdx.x < BM) sm.v1[0][threadIdx.x] = exp_acc(csQ - sm.cs[0][min(m0 + (int)threadIdx.x, d.Q - 1)]);
+        if (threadIdx.x < BM) {
+            const int s = min(m0 + (int)threadIdx.x, d.Q - 1);
+            sm.v1[0][threadIdx.x] = exp_acc(csQ - sm.cs[0][s]);
+            if (SEQ && sm.sid[s] != seq_end(d, b, c)) sm.v1[0][threadIdx.x] = 0.f;
+        }
         __syncthreads();
         const T* pbv = Bv.p + b * Bv.s0 + (int64_t)(l0 + m0) * Bv.s1 + g * Bv.s2;
         const bool kia = Bv.s1 == 1;
@@ -1157,7 +1213,7 @@ __global__ void __launch_bounds__(NTHR, TcEngine::MIN_CTAS) dx_kernel_tc(View4<T
 }
 
 // ---- B4: dCB[l][s] = sum_{h in g} dt'_s exp(cs_l - cs_s) (dout_h x_h^T)[l, s],  s <= l ------------
-template <typename T>
+template <typename T, bool SEQ>
 __global__ void __launch_bounds__(NTHR, 2) dcb_kernel(View4<T> X, View4<T> DO, Dims d, Ws ws, float* dcb, int x3) {
     Smem& sm = smem_ref();
     const int ntm = (d.Q + BM - 1) / BM, ntn = (d.Q + BN - 1) / BN;
@@ -1171,6 +1227,7 @@ __global__ void __launch_bounds__(NTHR, 2) dcb_kernel(View4<T> X, View4<T> DO, D
     const int m0 = tm * BM, s0 = tn * BN;
     if (m0 >= q || s0 >= q || s0 > m0 + BM - 1) return;
     const bool do_ifast = DO.s1 <= DO.s3, x_ifast = X.s1 <= X.s3;
+    if (SEQ) stage_sid(sm, d, b, c);   // read after the barrier of the first head's staging
     Acc tot;
     tot.zero();
     int buf = 0;
@@ -1202,7 +1259,7 @@ __global__ void __launch_bounds__(NTHR, 2) dcb_kernel(View4<T> X, View4<T> DO, D
 #pragma unroll
                 for (int r = 0; r < 4; ++r) {
                     const int l = m0 + wm0 + mi * 16 + gq + ((r & 2) ? 8 : 0), s = s0 + wn0 + ni * 8 + 2 * tq + (r & 1);
-                    if (l < q && s <= l) tot.v[mi][ni][r] += sm.dtp[hb][s] * exp_acc(sm.cs[hb][l] - sm.cs[hb][s]) * acc.v[mi][ni][r];
+                    if (l < q && s <= l && (!SEQ || sm.sid[l] == sm.sid[s])) tot.v[mi][ni][r] += sm.dtp[hb][s] * exp_acc(sm.cs[hb][l] - sm.cs[hb][s]) * acc.v[mi][ni][r];
                 }
     }
     float* o = dcb + (((size_t)b * d.nc + c) * d.G + g) * (size_t)d.Q * d.Q;
@@ -1213,7 +1270,7 @@ __global__ void __launch_bounds__(NTHR, 2) dcb_kernel(View4<T> X, View4<T> DO, D
 }
 
 // ---- B5: dC = dCB B + sum_h exp(cs_h) dout_h Sin_h ;  dB = dCB^T C + sum_h exp(cs_Q - cs) dt' x_h G_h ----
-template <typename T>
+template <typename T, bool SEQ>
 __global__ void __launch_bounds__(NTHR, 2) dbc_kernel(View4<T> X, View4<T> Bv, View4<T> Cv, View4<T> DO, Dims d, Ws ws,
                                                       const float* dcb_all, const float* G, float* dB, float* dC, OutS dbs, OutS dcs, int x3) {
     Smem& sm = smem_ref();
@@ -1267,6 +1324,9 @@ __global__ void __launch_bounds__(NTHR, 2) dbc_kernel(View4<T> X, View4<T> Bv, V
     const bool a_ifast = Asrc.s1 <= Asrc.s3;
     const float* Sbase = which == 0 ? ws.states : G;
     if (which == 0 || c + 1 < d.nc) {
+        // dC: only positions of the sequence entering the chunk see Sin; dB: only those of the sequence open at its end feed G
+        const int ref = SEQ ? (which == 0 ? seq_prev(d, b, c) : seq_end(d, b, c)) : 0;
+        if (SEQ) stage_sid(sm, d, b, c);
         for (int hh = 0; hh < d.hpg; ++hh) {
             const int h = g * d.hpg + hh, hb = hh & 1;
             stage_cs(sm, hb, ws, d, b, h, c);
@@ -1277,6 +1337,7 @@ __global__ void __launch_bounds__(NTHR, 2) dbc_kernel(View4<T> X, View4<T> Bv, V
                 fill_tile<BM, true>(sm.A[buf], a_ifast, [&](int i, int k) {
                     const int l = m0 + i, p = k0 + k;
                     if (l >= q || p >= d.P) return 0.f;
+                    if (SEQ && sm.sid[l] != ref) return 0.f;
                     const float w = which == 0 ? exp_acc(sm.cs[hb][l]) : exp_acc(csQ - sm.cs[hb][l]) * sm.dtp[hb][l];
                     return Asrc.at(b, l0 + l, h, p) * w;
                 });
@@ -1357,6 +1418,8 @@ __global__ void __launch_bounds__(NTHR, TcEngine::MIN_CTAS) dbc_kernel_tc(View4<
             if (threadIdx.x < BM) {   // the row factor, once per (head, row) instead of once per element
                 const int l = min(m0 + (int)threadIdx.x, d.Q - 1);
                 sm.v1[hb][threadIdx.x] = which == 0 ? exp_acc(sm.cs[hb][l]) : exp_acc(csQ - sm.cs[hb][l]) * sm.dtp[hb][l];
+                // dC: only positions of the sequence entering the chunk see Sin; dB: only those of the sequence open at its end feed G
+                if (d.seq.p && seq_at(d, b, c, l) != (which == 0 ? seq_prev(d, b, c) : seq_end(d, b, c))) sm.v1[hb][threadIdx.x] = 0.f;
             }
             __syncthreads();
             const float* S = Sbase + (((size_t)b * d.nc + c) * d.H + h) * (size_t)d.P * d.N;
@@ -1440,6 +1503,39 @@ __global__ void __launch_bounds__(MAXQ) dt_bwd_kernel(const T* dt, int64_t s0, i
     }
 }
 
+// ---- V1: state after the last token of each packed sequence (batch 1), after the forward -----------------------------
+// e = the sequence's last position, c its chunk:  S = sum_{s in [max(start, c Q), e]} exp(cs_e - cs_s) dt'_s x_s B_s^T
+//                                                   + exp(cs_e) Sin[c]   when the sequence began before chunk c (or at 0)
+// (mamba_ssm's chunk_state_varlen adds Sin[c] only when it began before chunk c, so it leaves initial_states out of a first
+// sequence that ends inside chunk 0; here that sequence includes them, as out and final_states do)
+// Grid (nseq, H, P N / 256); one thread per (p, n), SIMT over the at most Q tail positions.
+template <typename T>
+__global__ void __launch_bounds__(NTHR) varlen_states_kernel(View4<T> X, View4<T> Bv, Dims d, Ws ws, const int32_t* cu_seqlens, float* states) {
+    __shared__ float w[MAXQ];
+    const int k = blockIdx.x, h = blockIdx.y, g = h / d.hpg;
+    const int start = min(max(__ldg(cu_seqlens + k), 0), d.L), end = min(max(__ldg(cu_seqlens + k + 1), 0), d.L);
+    const int e = end - 1, c = max(e, 0) / d.Q, l0 = c * d.Q, s0 = max(start, l0);
+    const size_t csoff = ((size_t)h * d.nc + c) * d.Q;
+    const float cse = end > start ? ws.cs[csoff + e - l0] : 0.f;
+    for (int i = threadIdx.x; i < d.Q; i += NTHR) {
+        const int s = l0 + i;
+        w[i] = (s >= s0 && s <= e) ? exp_acc(cse - ws.cs[csoff + i]) * ws.dtp[csoff + i] : 0.f;
+    }
+    __syncthreads();
+    const int PN = d.P * d.N, idx = blockIdx.z * NTHR + threadIdx.x;
+    if (idx >= PN) return;
+    const int p = idx / d.N, n = idx % d.N;
+    float acc = 0.f;
+    if (end > start) {
+        // the chunk-entry state belongs to this sequence when it began before the chunk (or is the row's first); with seq_idx
+        // the forward's own mask decides, so out, final_states and these states agree
+        const bool entry = (start < l0 || start == 0) && (!d.seq.p || d.seq.at(0, e) == seq_prev(d, 0, c));
+        if (entry) acc = exp_acc(cse) * ws.states[((size_t)c * d.H + h) * PN + idx];
+        for (int s = s0; s <= e; ++s) acc = fmaf(w[s - l0] * X.at(0, s, h, p), Bv.at(0, s, g, n), acc);
+    }
+    states[((size_t)k * d.H + h) * PN + idx] = acc;
+}
+
 // ---- gated RMSNorm (SSD/MedSSD.py:393-394): y = rmsnorm(x silu(z)) w ------------------------------
 __device__ __forceinline__ float silu_f(float z) { return z / (1.f + expf(-z)); }
 
@@ -1516,6 +1612,9 @@ static int validate(const b200_ssd_fwd_params* p) {
     B200_REQUIRE(p->x && p->dt && p->A && p->B && p->C, "b200_ssd: x/dt/A/B/C must be non-NULL");
     B200_REQUIRE(p->workspace != nullptr, "b200_ssd: workspace is NULL");
     B200_REQUIRE((reinterpret_cast<uintptr_t>(p->workspace) & 15) == 0, "b200_ssd: workspace must be 16-byte aligned");
+    B200_REQUIRE(p->seq_idx == nullptr || (p->seq_idx_stride[0] >= 0 && p->seq_idx_stride[1] >= 0),
+                 "b200_ssd: seq_idx strides must be non-negative (got %lld, %lld)", (long long)p->seq_idx_stride[0],
+                 (long long)p->seq_idx_stride[1]);
     return 0;
 }
 
@@ -1547,6 +1646,42 @@ static bool use_tcgen05() {
     return on;
 }
 
+// K2 + K3: chunk states, then state passing (chunk-entry states and final_states)
+template <typename T, bool SEQ>
+static int states_fwd(const b200_ssd_fwd_params* p, const Dims& d, const Ws& ws, const View4<T>& X, const View4<T>& Bv, size_t smem, bool tcg,
+                      cudaStream_t st) {
+    const int x3 = p->precision == 0;
+    const size_t grid = (size_t)d.batch * d.nc * d.H * ((d.P + BN - 1) / BN) * ((d.N + BM - 1) / BM);
+    if (tcg) LAUNCH((chunk_state_kernel<T, 0, TcEngine, SEQ>), grid, NTHR, smem, st, X, Bv, d, ws, ws.states, x3);
+    else LAUNCH((chunk_state_kernel<T, 0, MmaEngine, SEQ>), grid, NTHR, smem, st, X, Bv, d, ws, ws.states, x3);
+    const size_t PN = (size_t)d.P * d.N;
+    const bool vec = PN % 4 == 0 && ((uintptr_t)ws.states & 15) == 0 && ((uintptr_t)p->initial_states & 15) == 0 &&
+                     ((uintptr_t)p->final_states & 15) == 0 && (size_t)d.batch * d.H <= 65535;
+    if (vec) {
+        state_pass_kernel<SEQ><<<dim3((unsigned)((PN / 4 + 255) / 256), (unsigned)(d.batch * d.H)), 256, 0, st>>>(d, ws, p->initial_states,
+                                                                                                         p->final_states);
+        if (int rc_ = check_launch("state_pass_kernel")) return rc_;
+    } else {
+        const size_t n = (size_t)d.batch * d.H * PN;
+        LAUNCH(state_pass_kernel_scalar<SEQ>, (n + 255) / 256, 256, 0, st, d, ws, p->initial_states, p->final_states);
+    }
+    return 0;
+}
+
+template <typename T, class E>
+static int chunk_scan(const b200_ssd_fwd_params* p, const Dims& d, const Ws& ws, const View4<T>& X, const View4<T>& Cv, size_t smem,
+                      cudaStream_t st) {
+    const size_t grid = (size_t)d.batch * d.nc * d.H * ((d.Q + BM - 1) / BM) * ((d.P + BN - 1) / BN);
+    const int x3 = p->precision == 0, has_init = p->initial_states != nullptr;
+    if (d.seq.p)
+        LAUNCH((chunk_scan_kernel<T, E, true>), grid, NTHR, smem, st, X, Cv, p->D, d, ws, (T*)p->out, p->out_stride[0], p->out_stride[1],
+               p->out_stride[2], p->out_stride[3], has_init, x3);
+    else
+        LAUNCH((chunk_scan_kernel<T, E, false>), grid, NTHR, smem, st, X, Cv, p->D, d, ws, (T*)p->out, p->out_stride[0], p->out_stride[1],
+               p->out_stride[2], p->out_stride[3], has_init, x3);
+    return 0;
+}
+
 template <typename T>
 static int fwd_impl(const b200_ssd_fwd_params* p, cudaStream_t st) {
     const Dims d = make_dims(*p);
@@ -1555,36 +1690,21 @@ static int fwd_impl(const b200_ssd_fwd_params* p, cudaStream_t st) {
     const int x3 = p->precision == 0;
     const size_t SM = sizeof(Smem);
     const int ntq128 = (d.Q + BM - 1) / BM, ntq64 = (d.Q + BN - 1) / BN;
-    const int ntn128 = (d.N + BM - 1) / BM, ntp64 = (d.P + BN - 1) / BN;
     LAUNCH((dt_cumsum_kernel<T>), (size_t)d.batch * d.H * d.nc, d.Q, 0, st, (const T*)p->dt, p->dt_stride[0], p->dt_stride[1],
            p->dt_stride[2], p->A, p->dt_bias, p->dt_softplus, p->dt_min, p->dt_max, d, ws);
     const bool tcg = use_tcgen05();
     const size_t SMT = x3 ? tc::SMEM_X3 : tc::SMEM_TF32;
-    if (tcg) LAUNCH((chunk_state_kernel<T, 0, TcEngine>), (size_t)d.batch * d.nc * d.H * ntp64 * ntn128, NTHR, SMT, st, X, Bv, d, ws, ws.states, x3);
-    else LAUNCH((chunk_state_kernel<T, 0, MmaEngine>), (size_t)d.batch * d.nc * d.H * ntp64 * ntn128, NTHR, SM, st, X, Bv, d, ws, ws.states, x3);
-    {
-        const size_t PN = (size_t)d.P * d.N;
-        const bool vec = PN % 4 == 0 && ((uintptr_t)ws.states & 15) == 0 && ((uintptr_t)p->initial_states & 15) == 0 &&
-                         ((uintptr_t)p->final_states & 15) == 0 && (size_t)d.batch * d.H <= 65535;
-        if (vec) {
-            state_pass_kernel<<<dim3((unsigned)((PN / 4 + 255) / 256), (unsigned)(d.batch * d.H)), 256, 0, st>>>(d, ws, p->initial_states,
-                                                                                                            p->final_states);
-            if (int rc_ = check_launch("state_pass_kernel")) return rc_;
-        } else {
-            const size_t n = (size_t)d.batch * d.H * PN;
-            LAUNCH(state_pass_kernel_scalar, (n + 255) / 256, 256, 0, st, d, ws, p->initial_states, p->final_states);
-        }
+    if (d.seq.p) {
+        if (int rc = states_fwd<T, true>(p, d, ws, X, Bv, tcg ? SMT : SM, tcg, st)) return rc;
+    } else {
+        if (int rc = states_fwd<T, false>(p, d, ws, X, Bv, tcg ? SMT : SM, tcg, st)) return rc;
     }
     if (tcg) {
         LAUNCH((cb_kernel<T, TcEngine>), (size_t)d.batch * d.nc * d.G * ntq128 * ntq64, NTHR, SMT, st, Cv, Bv, d, ws, x3);
-        LAUNCH((chunk_scan_kernel<T, TcEngine>), (size_t)d.batch * d.nc * d.H * ntq128 * ntp64, NTHR, SMT, st, X, Cv, p->D, d, ws, (T*)p->out,
-               p->out_stride[0], p->out_stride[1], p->out_stride[2], p->out_stride[3], p->initial_states != nullptr, x3);
-    } else {
-        LAUNCH((cb_kernel<T, MmaEngine>), (size_t)d.batch * d.nc * d.G * ntq128 * ntq64, NTHR, SM, st, Cv, Bv, d, ws, x3);
-        LAUNCH((chunk_scan_kernel<T, MmaEngine>), (size_t)d.batch * d.nc * d.H * ntq128 * ntp64, NTHR, SM, st, X, Cv, p->D, d, ws, (T*)p->out,
-               p->out_stride[0], p->out_stride[1], p->out_stride[2], p->out_stride[3], p->initial_states != nullptr, x3);
+        return chunk_scan<T, TcEngine>(p, d, ws, X, Cv, SMT, st);
     }
-    return 0;
+    LAUNCH((cb_kernel<T, MmaEngine>), (size_t)d.batch * d.nc * d.G * ntq128 * ntq64, NTHR, SM, st, Cv, Bv, d, ws, x3);
+    return chunk_scan<T, MmaEngine>(p, d, ws, X, Cv, SM, st);
 }
 
 struct Scratch {
@@ -1607,6 +1727,51 @@ static Scratch make_scratch(float* base, const Dims& d) {
     return s;
 }
 
+// B1 - B5 (B6, dt_bwd_kernel, needs no mask: the masked terms are already absent from its inputs)
+template <typename T, bool SEQ>
+static int bwd_masked(const b200_ssd_bwd_params* q, const Dims& d, const Ws& ws, const Scratch& sc, const View4<T>& X, const View4<T>& Bv,
+                      const View4<T>& Cv, const View4<T>& DO, const View4<T>& OUT, const OutS& dxs, const OutS& dbs, const OutS& dcs,
+                      cudaStream_t st) {
+    const b200_ssd_fwd_params* p = &q->f;
+    const int x3 = p->precision == 0;
+    const size_t SM = sizeof(Smem);
+    const int ntq128 = (d.Q + BM - 1) / BM, ntq64 = (d.Q + BN - 1) / BN;
+    const int ntn128 = (d.N + BM - 1) / BM, ntn64 = (d.N + BN - 1) / BN, ntp64 = (d.P + BN - 1) / BN;
+    if (use_tcgen05())
+        LAUNCH((chunk_state_kernel<T, 1, TcEngine, SEQ>), (size_t)d.batch * d.nc * d.H * ntp64 * ntn128, NTHR, (x3 ? tc::SMEM_X3 : tc::SMEM_TF32),
+               st, DO, Cv, d, ws, sc.dstates, x3);
+    else
+        LAUNCH((chunk_state_kernel<T, 1, MmaEngine, SEQ>), (size_t)d.batch * d.nc * d.H * ntp64 * ntn128, NTHR, SM, st, DO, Cv, d, ws, sc.dstates,
+               x3);
+    {
+        const size_t PN = (size_t)d.P * d.N;
+        const bool vec = PN % 4 == 0 && ((uintptr_t)ws.states & 15) == 0 && ((uintptr_t)sc.dstates & 15) == 0 &&
+                         (size_t)d.batch * d.H <= 65535;
+        if (vec) {
+            state_pass_bwd_kernel<SEQ><<<dim3((unsigned)((PN / 4 + NTHR - 1) / NTHR), (unsigned)(d.batch * d.H)), NTHR, 0, st>>>(d, ws, sc.dstates,
+                                                                                                                        sc.dcsQ);
+            if (int rc_ = check_launch("state_pass_bwd_kernel")) return rc_;
+        } else {
+            const int nblk = (int)((PN + NTHR - 1) / NTHR);
+            LAUNCH(state_pass_bwd_kernel_scalar<SEQ>, (size_t)d.batch * d.H * nblk, NTHR, 0, st, d, ws, sc.dstates, sc.dcsQ);
+        }
+    }
+    if (use_tcgen05())
+        LAUNCH((dx_kernel_tc<T, SEQ>), (size_t)d.batch * d.nc * d.H * ntq128 * ntp64, NTHR, (x3 ? tc::SMEM_X3 : tc::SMEM_TF32), st, X, Bv, DO, OUT,
+               p->D, d, ws, sc.dstates, q->dx, dxs, sc.ddtp_exp, sc.dcs_pos, q->dD, x3);
+    else
+        LAUNCH((dx_kernel<T, SEQ>), (size_t)d.batch * d.nc * d.H * ntq128 * ntp64, NTHR, SM, st, X, Bv, DO, OUT, p->D, d, ws, sc.dstates, q->dx,
+               dxs, sc.ddtp_exp, sc.dcs_pos, q->dD, x3);
+    LAUNCH((dcb_kernel<T, SEQ>), (size_t)d.batch * d.nc * d.G * ntq128 * ntq64, NTHR, SM, st, X, DO, d, ws, sc.dcb, x3);
+    if (use_tcgen05())
+        LAUNCH((dbc_kernel_tc<T>), (size_t)d.batch * d.nc * d.G * ntq128 * ntn64 * 2, NTHR, (x3 ? tc::SMEM_X3 : tc::SMEM_TF32), st, X, Bv, Cv, DO, d,
+               ws, sc.dcb, sc.dstates, q->dB, q->dC, dbs, dcs, x3);
+    else
+        LAUNCH((dbc_kernel<T, SEQ>), (size_t)d.batch * d.nc * d.G * ntq128 * ntn64 * 2, NTHR, SM, st, X, Bv, Cv, DO, d, ws, sc.dcb, sc.dstates,
+               q->dB, q->dC, dbs, dcs, x3);
+    return 0;
+}
+
 template <typename T>
 static int bwd_impl(const b200_ssd_bwd_params* q, cudaStream_t st) {
     const b200_ssd_fwd_params* p = &q->f;
@@ -1615,10 +1780,6 @@ static int bwd_impl(const b200_ssd_bwd_params* q, cudaStream_t st) {
     const Scratch sc = make_scratch(q->scratch, d);
     const View4<T> X = view4<T>(p->x, p->x_stride), Bv = view4<T>(p->B, p->B_stride), Cv = view4<T>(p->C, p->C_stride);
     const View4<T> DO = view4<T>(q->dout, q->dout_stride), OUT = view4<T>(p->out, p->out_stride);
-    const int x3 = p->precision == 0;
-    const size_t SM = sizeof(Smem);
-    const int ntq128 = (d.Q + BM - 1) / BM, ntq64 = (d.Q + BN - 1) / BN;
-    const int ntn128 = (d.N + BM - 1) / BM, ntn64 = (d.N + BN - 1) / BN, ntp64 = (d.P + BN - 1) / BN;
     const OutS dxs = outs_of(q->dx_stride, d.L, d.H, d.P), dbs = outs_of(q->dB_stride, d.L, d.G, d.N), dcs = outs_of(q->dC_stride, d.L, d.G, d.N);
     const int64_t dt3[4] = {q->ddt_stride[0], q->ddt_stride[1], q->ddt_stride[2], 0};
     const OutS dts = outs_of(dt3, d.L, d.H, 1);
@@ -1627,37 +1788,11 @@ static int bwd_impl(const b200_ssd_bwd_params* q, cudaStream_t st) {
         set_error("b200_ssd_bwd: cudaMemsetAsync: %s", cudaGetErrorString(e));
         return (int)e;
     }
-    if (use_tcgen05())
-        LAUNCH((chunk_state_kernel<T, 1, TcEngine>), (size_t)d.batch * d.nc * d.H * ntp64 * ntn128, NTHR, (x3 ? tc::SMEM_X3 : tc::SMEM_TF32), st,
-               DO, Cv, d, ws, sc.dstates, x3);
-    else
-        LAUNCH((chunk_state_kernel<T, 1, MmaEngine>), (size_t)d.batch * d.nc * d.H * ntp64 * ntn128, NTHR, SM, st, DO, Cv, d, ws, sc.dstates, x3);
-    {
-        const size_t PN = (size_t)d.P * d.N;
-        const bool vec = PN % 4 == 0 && ((uintptr_t)ws.states & 15) == 0 && ((uintptr_t)sc.dstates & 15) == 0 &&
-                         (size_t)d.batch * d.H <= 65535;
-        if (vec) {
-            state_pass_bwd_kernel<<<dim3((unsigned)((PN / 4 + NTHR - 1) / NTHR), (unsigned)(d.batch * d.H)), NTHR, 0, st>>>(d, ws, sc.dstates,
-                                                                                                                   sc.dcsQ);
-            if (int rc_ = check_launch("state_pass_bwd_kernel")) return rc_;
-        } else {
-            const int nblk = (int)((PN + NTHR - 1) / NTHR);
-            LAUNCH(state_pass_bwd_kernel_scalar, (size_t)d.batch * d.H * nblk, NTHR, 0, st, d, ws, sc.dstates, sc.dcsQ);
-        }
+    if (d.seq.p) {
+        if (int rc = bwd_masked<T, true>(q, d, ws, sc, X, Bv, Cv, DO, OUT, dxs, dbs, dcs, st)) return rc;
+    } else {
+        if (int rc = bwd_masked<T, false>(q, d, ws, sc, X, Bv, Cv, DO, OUT, dxs, dbs, dcs, st)) return rc;
     }
-    if (use_tcgen05())
-        LAUNCH((dx_kernel_tc<T>), (size_t)d.batch * d.nc * d.H * ntq128 * ntp64, NTHR, (x3 ? tc::SMEM_X3 : tc::SMEM_TF32), st, X, Bv, DO, OUT, p->D,
-               d, ws, sc.dstates, q->dx, dxs, sc.ddtp_exp, sc.dcs_pos, q->dD, x3);
-    else
-        LAUNCH((dx_kernel<T>), (size_t)d.batch * d.nc * d.H * ntq128 * ntp64, NTHR, SM, st, X, Bv, DO, OUT, p->D, d, ws, sc.dstates, q->dx, dxs,
-               sc.ddtp_exp, sc.dcs_pos, q->dD, x3);
-    LAUNCH((dcb_kernel<T>), (size_t)d.batch * d.nc * d.G * ntq128 * ntq64, NTHR, SM, st, X, DO, d, ws, sc.dcb, x3);
-    if (use_tcgen05())
-        LAUNCH((dbc_kernel_tc<T>), (size_t)d.batch * d.nc * d.G * ntq128 * ntn64 * 2, NTHR, (x3 ? tc::SMEM_X3 : tc::SMEM_TF32), st, X, Bv, Cv, DO, d,
-               ws, sc.dcb, sc.dstates, q->dB, q->dC, dbs, dcs, x3);
-    else
-        LAUNCH((dbc_kernel<T>), (size_t)d.batch * d.nc * d.G * ntq128 * ntn64 * 2, NTHR, SM, st, X, Bv, Cv, DO, d, ws, sc.dcb, sc.dstates,
-               q->dB, q->dC, dbs, dcs, x3);
     LAUNCH((dt_bwd_kernel<T>), (size_t)d.batch * d.H * d.nc, d.Q, 0, st, (const T*)p->dt, p->dt_stride[0], p->dt_stride[1],
            p->dt_stride[2], p->A, p->dt_bias, p->dt_softplus, p->dt_min, p->dt_max, d, ws, sc.ddtp_exp, sc.dcs_pos, sc.dcsQ, q->ddt, dts,
            q->dA, q->ddt_bias);
@@ -1678,6 +1813,7 @@ static Dims dims_of(int32_t batch, int32_t seqlen, int32_t nheads, int32_t headd
     d.batch = batch; d.L = seqlen; d.H = nheads; d.P = headdim; d.G = n_groups; d.N = dstate; d.Q = chunk;
     d.nc = (seqlen + chunk - 1) / chunk;
     d.hpg = nheads / n_groups;
+    d.seq = Seq{nullptr, 0, 0};
     return d;
 }
 
@@ -1719,6 +1855,32 @@ extern "C" int b200_ssd_bwd(const b200_ssd_bwd_params* q, b200_stream_t stream) 
         case B200_BF16: return bwd_impl<__nv_bfloat16>(q, st);
         default: return bwd_impl<__half>(q, st);
     }
+}
+
+extern "C" int b200_ssd_varlen_states(const b200_ssd_fwd_params* p, const int32_t* cu_seqlens, int32_t nseq, float* states,
+                                      b200_stream_t stream) {
+    if (int rc = ssd::validate(p)) return rc;
+    B200_REQUIRE(p->batch == 1, "b200_ssd_varlen_states: packed sequences need batch == 1 (got %d)", p->batch);
+    B200_REQUIRE(cu_seqlens && states, "b200_ssd_varlen_states: cu_seqlens / states must be non-NULL");
+    B200_REQUIRE(nseq >= 1 && nseq <= 65535, "b200_ssd_varlen_states: nseq %d must be in [1, 65535]", nseq);
+    B200_REQUIRE(p->nheads <= 65535, "b200_ssd_varlen_states: nheads %d > 65535", p->nheads);
+    const Dims d = make_dims(*p);
+    const Ws ws = make_ws(p->workspace, d);
+    const dim3 grid((unsigned)nseq, (unsigned)d.H, (unsigned)((d.P * d.N + NTHR - 1) / NTHR));
+    cudaStream_t st = (cudaStream_t)stream;
+    switch (p->io_dtype) {
+        case B200_F32:
+            varlen_states_kernel<float><<<grid, NTHR, 0, st>>>(view4<float>(p->x, p->x_stride), view4<float>(p->B, p->B_stride), d, ws, cu_seqlens, states);
+            break;
+        case B200_BF16:
+            varlen_states_kernel<__nv_bfloat16><<<grid, NTHR, 0, st>>>(view4<__nv_bfloat16>(p->x, p->x_stride), view4<__nv_bfloat16>(p->B, p->B_stride),
+                                                                      d, ws, cu_seqlens, states);
+            break;
+        default:
+            varlen_states_kernel<__half><<<grid, NTHR, 0, st>>>(view4<__half>(p->x, p->x_stride), view4<__half>(p->B, p->B_stride), d, ws, cu_seqlens,
+                                                               states);
+    }
+    return check_launch("varlen_states_kernel");
 }
 
 extern "C" int b200_rmsnorm_gated_fwd(const float* x, const float* z, const float* w, float* y, float* rstd, int64_t rows, int32_t dim,

@@ -7,13 +7,20 @@
 
 x (batch, L, H, P); dt (batch, L, H); A (H); B, C (batch, L, G, N); D (H) or (H, P); z like x;
 dt_bias (H); initial_states (batch, H, P, N).  Returns out (batch, L, H, P) in x's dtype
-[, final_states (batch, H, P, N) fp32].  Tensors are taken with whatever strides they have (the
-reference passes (b, l, .) views of channel-major storage, L stride 1) -- nothing is copied.
+[, final_states (batch, H, P, N) fp32][, varlen_states (nseq, H, P, N) fp32].  Tensors are taken with
+whatever strides they have (the reference passes (b, l, .) views of channel-major storage, L stride 1)
+-- nothing is copied.
+
+Packed sequences: seq_idx (batch, L) integers, non-decreasing along L (the caller's contract, not
+checked: that would need a host sync), restarts the recurrence wherever it changes, in the forward
+and in the backward; initial_states[b] reach row b's first sequence only when its id is 0.
+return_varlen_states (batch 1, cu_seqlens (nseq + 1,) giving the same boundaries) also returns the
+state after each sequence's last token.  It differs from mamba_ssm in one case: a first sequence that
+ends inside the first chunk includes initial_states, as out and final_states do.
 
 The work is done by libb200ssm.so (csrc/ssd.cu, sm_100a tensor-core kernels) through its C ABI
-(include/b200_ssm.h: b200_ssd_fwd / b200_ssd_bwd).  There is no CPU path: CPU tensors raise.
-`seq_idx` / `cu_seqlens` (variable-length batches) are never passed by the reference models and
-raise NotImplementedError.
+(include/b200_ssm.h: b200_ssd_fwd / b200_ssd_bwd / b200_ssd_varlen_states).  There is no CPU path:
+CPU tensors raise.
 """
 from __future__ import annotations
 
@@ -61,7 +68,7 @@ def set_precision(mode) -> None:
     _explicit = True
 
 
-def _fill_fwd(p, x, dt, A, Bm, Cm, D, dt_bias, chunk_size, dt_softplus, dt_limit, initial_states, precision):
+def _fill_fwd(p, x, dt, A, Bm, Cm, D, dt_bias, chunk_size, dt_softplus, dt_limit, initial_states, precision, seq_idx):
     batch, L, H, P = x.shape
     G, N = Bm.shape[2], Bm.shape[3]
     p.batch, p.seqlen, p.nheads, p.headdim, p.n_groups, p.dstate, p.chunk_size = batch, L, H, P, G, N, chunk_size
@@ -74,6 +81,9 @@ def _fill_fwd(p, x, dt, A, Bm, Cm, D, dt_bias, chunk_size, dt_softplus, dt_limit
     p.dt_stride[:] = list(dt.stride())
     p.x, p.dt, p.A, p.B, p.C = x.data_ptr(), dt.data_ptr(), A.data_ptr(), Bm.data_ptr(), Cm.data_ptr()
     p.D, p.dt_bias, p.initial_states = _lib.ptr(D), _lib.ptr(dt_bias), _lib.ptr(initial_states)
+    if seq_idx is not None:
+        p.seq_idx = seq_idx.data_ptr()
+        p.seq_idx_stride[:] = list(seq_idx.stride())
 
 
 def _empty_like_layout(t):
@@ -86,7 +96,8 @@ def _empty_like_layout(t):
 class SsdChunkScanFn(torch.autograd.Function):
     @staticmethod
     @_no_autocast
-    def forward(ctx, x, dt, A, B, C, D, dt_bias, initial_states, chunk_size, dt_softplus, dt_limit, return_final_states, prec):
+    def forward(ctx, x, dt, A, B, C, D, dt_bias, initial_states, seq_idx, cu_seqlens, chunk_size, dt_softplus, dt_limit,
+                return_final_states, prec):
         batch, L, H, P = x.shape
         G, N = B.shape[2], B.shape[3]
         dev = x.device
@@ -97,7 +108,7 @@ class SsdChunkScanFn(torch.autograd.Function):
         nbytes = _lib.load().b200_ssd_workspace_bytes(batch, L, H, P, G, N, chunk_size)
         ws = torch.empty(nbytes // 4, dtype=torch.float32, device=dev)
         p = _lib.SsdFwdParams()
-        _fill_fwd(p, x, dt_, A32, B_, C_, D32, bias32, chunk_size, dt_softplus, dt_limit, init32, prec)
+        _fill_fwd(p, x, dt_, A32, B_, C_, D32, bias32, chunk_size, dt_softplus, dt_limit, init32, prec, seq_idx)
         p.out_stride[:] = list(out.stride())
         p.out, p.final_states, p.workspace = out.data_ptr(), _lib.ptr(fin), ws.data_ptr()
         prof = _profiler
@@ -106,19 +117,26 @@ class SsdChunkScanFn(torch.autograd.Function):
             _lib.launch("b200_ssd_fwd", dev, ctypes.byref(p))
             if prof is not None:
                 prof.end(tok, "fwd", (batch, L, H, P, G, N, chunk_size, prec))
-        ctx.save_for_backward(x, dt_, A32, B_, C_, D32, bias32, init32, out, ws)
+        extra = (fin,) if return_final_states else ()
+        if cu_seqlens is not None:      # return_varlen_states: reads this call's workspace
+            nseq = cu_seqlens.shape[0] - 1
+            varlen = torch.empty((nseq, H, P, N), dtype=torch.float32, device=dev)
+            if nseq > 0:
+                _lib.launch("b200_ssd_varlen_states", dev, ctypes.byref(p), cu_seqlens.data_ptr(), nseq, varlen.data_ptr())
+            extra += (varlen,)
+        ctx.save_for_backward(x, dt_, A32, B_, C_, D32, bias32, init32, seq_idx, out, ws)
         ctx.cfg = (chunk_size, bool(dt_softplus), tuple(dt_limit), prec)
         ctx.dtypes = (dt.dtype, A.dtype, B.dtype, C.dtype, None if D is None else D.dtype,
                       None if dt_bias is None else dt_bias.dtype)
-        if return_final_states:
-            ctx.mark_non_differentiable(fin)
-            return out, fin
+        if extra:
+            ctx.mark_non_differentiable(*extra)
+            return (out,) + extra
         return out
 
     @staticmethod
     @_no_autocast
     def backward(ctx, dout, *unused):
-        x, dt_, A32, B_, C_, D32, bias32, init32, out, ws = ctx.saved_tensors
+        x, dt_, A32, B_, C_, D32, bias32, init32, seq_idx, out, ws = ctx.saved_tensors
         chunk_size, dt_softplus, dt_limit, precision = ctx.cfg
         batch, L, H, P = x.shape
         G, N = B_.shape[2], B_.shape[3]
@@ -133,7 +151,7 @@ class SsdChunkScanFn(torch.autograd.Function):
         nbytes = _lib.load().b200_ssd_bwd_scratch_bytes(batch, L, H, P, G, N, chunk_size)
         scratch = torch.empty(nbytes // 4, dtype=torch.float32, device=dev)
         q = _lib.SsdBwdParams()
-        _fill_fwd(q.f, x, dt_, A32, B_, C_, D32, bias32, chunk_size, dt_softplus, dt_limit, init32, precision)
+        _fill_fwd(q.f, x, dt_, A32, B_, C_, D32, bias32, chunk_size, dt_softplus, dt_limit, init32, precision, seq_idx)
         q.f.out_stride[:] = list(out.stride())
         q.f.out, q.f.workspace = out.data_ptr(), ws.data_ptr()
         q.dout_stride[:] = list(dout.stride())
@@ -150,7 +168,7 @@ class SsdChunkScanFn(torch.autograd.Function):
         t_dt, t_A, t_B, t_C, t_D, t_bias = ctx.dtypes
         return (dx.to(x.dtype), ddt.to(t_dt), dA.to(t_A), dB.to(t_B), dC.to(t_C),
                 None if dD is None else dD.to(t_D), None if dbias is None else dbias.to(t_bias),
-                None, None, None, None, None, None)
+                None, None, None, None, None, None, None, None)
 
 
 def mamba_chunk_scan_combined(x, dt, A, B, C, chunk_size, D=None, z=None, dt_bias=None, initial_states=None,
@@ -161,14 +179,15 @@ def mamba_chunk_scan_combined(x, dt, A, B, C, chunk_size, D=None, z=None, dt_bia
         B, C: (batch, seqlen, ngroups, dstate)  chunk_size: int
         D: (nheads, headdim) or (nheads,)       z: (batch, seqlen, nheads, headdim)
         dt_bias: (nheads,)                      initial_states: (batch, nheads, headdim, dstate)
+        seq_idx: (batch, seqlen) integers, non-decreasing along seqlen: the recurrence restarts where it changes
+        cu_seqlens: (nseq + 1,) integers, sequence boundaries of the packed row; used by return_varlen_states (batch 1)
         dt_softplus: whether to apply softplus to dt
     Return:
         out: (batch, seqlen, nheads, headdim) [, final_states (batch, nheads, headdim, dstate)]
+        [, varlen_states (nseq, nheads, headdim, dstate): the state after each sequence's last token]
+    final_states and varlen_states are fp32 and carry no gradient.
     """
-    if seq_idx is not None or cu_seqlens is not None or return_varlen_states:
-        raise NotImplementedError("mamba_chunk_scan_combined: seq_idx / cu_seqlens (variable-length batches) are not "
-                                  "supported by the B200 kernels (never passed by the reference models)")
-    _lib.require_cuda(x, dt, A, B, C, D, z, dt_bias, initial_states)
+    _lib.require_cuda(x, dt, A, B, C, D, z, dt_bias, initial_states, seq_idx)
     if x.dim() != 4 or dt.dim() != 3 or B.dim() != 4 or C.dim() != 4:
         raise RuntimeError(f"mamba_chunk_scan_combined: expected x (b,l,h,p), dt (b,l,h), B/C (b,l,g,n); got "
                            f"{tuple(x.shape)}, {tuple(dt.shape)}, {tuple(B.shape)}, {tuple(C.shape)}")
@@ -185,6 +204,17 @@ def mamba_chunk_scan_combined(x, dt, A, B, C, chunk_size, D=None, z=None, dt_bia
             raise RuntimeError(f"mamba_chunk_scan_combined: initial_states must be {(batch, H, P, N)}")
         if initial_states.requires_grad:
             raise NotImplementedError("mamba_chunk_scan_combined: no gradient for initial_states in the B200 kernels")
+    seq_idx = _index_tensor(seq_idx, "seq_idx", x.device, (batch, L))
+    if return_varlen_states:
+        if cu_seqlens is None:
+            raise RuntimeError("mamba_chunk_scan_combined: return_varlen_states needs cu_seqlens")
+        if batch != 1:
+            raise RuntimeError(f"mamba_chunk_scan_combined: return_varlen_states needs batch == 1 (packed sequences), got {batch}")
+        if cu_seqlens.dim() != 1 or cu_seqlens.shape[0] < 1:
+            raise RuntimeError(f"mamba_chunk_scan_combined: cu_seqlens must be 1-D (nseq + 1,), got {tuple(cu_seqlens.shape)}")
+        cu_seqlens = _index_tensor(cu_seqlens, "cu_seqlens", x.device, tuple(cu_seqlens.shape))
+    else:
+        cu_seqlens = None          # accepted and unused, as in mamba_ssm
     D_head = None
     if D is not None:
         if tuple(D.shape) == (H,):
@@ -198,15 +228,30 @@ def mamba_chunk_scan_combined(x, dt, A, B, C, chunk_size, D=None, z=None, dt_bia
     # so every chunk_size mamba_ssm accepts (any power of two >= 16; the reference passes 256, SSD/MedSSD.py:365) is honoured by
     # running the kernels on the nearest length they tile: a multiple of 32 in [32, 256].
     chunk_size = min(256, (chunk_size + 31) // 32 * 32)
-    res = SsdChunkScanFn.apply(x, dt, A, B, C, D_head, dt_bias, initial_states, chunk_size, dt_softplus,
+    res = SsdChunkScanFn.apply(x, dt, A, B, C, D_head, dt_bias, initial_states, seq_idx, cu_seqlens, chunk_size, dt_softplus,
                                (float(dt_limit[0]), float(dt_limit[1])), return_final_states,
                                _effective_precision())   # read here: autocast is off inside the Function
-    out, fin = res if return_final_states else (res, None)
+    out, extra = (res[0], res[1:]) if isinstance(res, tuple) else (res, ())
     if D is not None and D_head is None:      # D with a head dimension: plain PyTorch on the side (unused by the models)
         out = out + x * D.to(x.dtype)
     if z is not None:                         # out * silu(z), as mamba_ssm does when no norm is fused
         out = out * F.silu(z)
-    return (out, fin) if return_final_states else out
+    return (out,) + extra if extra else out
+
+
+def _index_tensor(t, name, device, shape):
+    """t as the int32 tensor the kernels read (in place when it already is int32 with a unit last stride); None stays None."""
+    if t is None:
+        return None
+    if t.dtype.is_floating_point or t.dtype.is_complex or t.dtype == torch.bool:
+        raise RuntimeError(f"mamba_chunk_scan_combined: {name} must hold integers, got {t.dtype}")
+    if tuple(t.shape) != shape:
+        raise RuntimeError(f"mamba_chunk_scan_combined: {name} must be {shape}, got {tuple(t.shape)}")
+    if t.device != device:
+        raise RuntimeError(f"mamba_chunk_scan_combined: {name} is on {t.device}, x on {device}")
+    if t.dtype != torch.int32 or (t.shape[-1] > 1 and t.stride(-1) != 1):
+        t = t.to(torch.int32).contiguous()
+    return t
 
 
 # ------------------------------------------------------------------------------------------------
