@@ -248,7 +248,7 @@ typedef struct {
 } b200_ssd_fwd_params;
 
 typedef struct {
-    b200_ssd_fwd_params f;  /* forward inputs + its workspace (f.out / f.final_states unused) */
+    b200_ssd_fwd_params f;  /* forward inputs, its output f.out and its workspace (f.final_states unused: see final_states below) */
     int64_t dout_stride[4];
     const void* dout;
     /* gradients: fp32 in the logical shapes of their primals (strides below), written (not accumulated)
@@ -268,6 +268,14 @@ typedef struct {
     int64_t ddt_stride[3];
     int64_t dB_stride[4];
     int64_t dC_stride[4];
+    /* state gradients, (batch, H, P, N) contiguous f32, each NULL unless requested.  dfinal_states is the adjoint of the state
+       after each row's last token (with seq_idx it reaches the row's last sequence only) and needs final_states, the forward's
+       final_states output.  dinitial_states (written, not accumulated) needs f.initial_states; with seq_idx, a row whose first
+       id is not 0 gets zeros.  With both NULL the backward runs exactly as without them.  A rule broken returns an error and
+       launches nothing. */
+    const float* final_states;
+    const float* dfinal_states;
+    float* dinitial_states;
 } b200_ssd_bwd_params;
 
 size_t b200_ssd_workspace_bytes(int32_t batch, int32_t seqlen, int32_t nheads, int32_t headdim,

@@ -70,6 +70,7 @@ class SsdBwdParams(C.Structure):
         ("dout", vp), ("dx", vp), ("ddt", vp), ("dB", vp), ("dC", vp), ("dA", vp), ("dD", vp),
         ("ddt_bias", vp), ("scratch", vp),
         ("dx_stride", i64 * 4), ("ddt_stride", i64 * 3), ("dB_stride", i64 * 4), ("dC_stride", i64 * 4),
+        ("final_states", vp), ("dfinal_states", vp), ("dinitial_states", vp),
     ]
 
 

@@ -53,7 +53,7 @@ cudaError_t func_attr_per_device(const void* kernel, cudaFuncAttribute attr, int
 }  // namespace b200
 
 extern "C" const char* b200_last_error(void) { return b200::g_err; }
-extern "C" int b200_version(void) { return 2; }
+extern "C" int b200_version(void) { return 3; }
 extern "C" int b200_kernel_launches(void) { return b200::g_launches.load(std::memory_order_relaxed); }
 extern "C" size_t b200_sizeof_params(int32_t which) {
     switch (which) {

@@ -931,8 +931,13 @@ __global__ void __launch_bounds__(NTHR, E::MIN_CTAS) chunk_scan_kernel(View4<T> 
 //          dcsQ[b][h][c] = <G[c], Sin[c+1]>  (accumulated with atomics; caller zero-fills) ----------
 // Same streaming structure as K3 (128-bit, 8 chunks of loads in flight); the per-chunk dot products are kept in
 // registers and block-reduced once per batch of chunks.
+// State gradients (each NULL unless the caller asks): dfin seeds G[nc-1] (otherwise zero, and its dcsQ term, whose
+// Sin[nc] is the forward's final states fin, is skipped); dinit receives the adjoint of Sin[0] left after chunk 0.
+// With seq_idx the existing masks confine both: dec[0] = 0 when a sequence starts in chunk 0, and B1 keeps only
+// the positions of id 0 in chunk 0's off-diagonal adjoint.
 template <bool SEQ>
-__global__ void __launch_bounds__(NTHR) state_pass_bwd_kernel(Dims d, Ws ws, float* dstates, float* dcsQ) {
+__global__ void __launch_bounds__(NTHR) state_pass_bwd_kernel(Dims d, Ws ws, float* dstates, float* dcsQ, const float* fin,
+                                                              const float* dfin, float* dinit) {
     __shared__ float red[NTHR / 32][SPB];
     const int PN4 = d.P * d.N / 4;
     const int e = blockIdx.x * blockDim.x + threadIdx.x;
@@ -943,8 +948,28 @@ __global__ void __launch_bounds__(NTHR) state_pass_bwd_kernel(Dims d, Ws ws, flo
     const float4* sn = reinterpret_cast<const float4*>(ws.states) + ((size_t)b * d.nc * d.H + h) * PN4 + (ok ? e : 0);
     const float* csq = ws.cs + ((size_t)b * d.H + h) * d.nc * d.Q + d.Q - 1;
     float* dq = dcsQ + ((size_t)b * d.H + h) * d.nc;
-    float4 run = make_float4(0.f, 0.f, 0.f, 0.f);
+    const size_t bh4 = ((size_t)b * d.H + h) * PN4 + (ok ? e : 0);   // this thread's float4 of a (batch, H, P, N) tensor
     const float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
+    float4 run = z4;
+    if (dfin) {   // G[nc-1] = dfin and its term dcsQ[nc-1] = <dfin, fin>, before the loop so that the loop keeps its registers
+        float dot = 0.f;
+        if (ok) {
+            run = reinterpret_cast<const float4*>(dfin)[bh4];
+            const float4 f = reinterpret_cast<const float4*>(fin)[bh4];
+            dot = run.x * f.x + run.y * f.y + run.z * f.z + run.w * f.w;
+        }
+#pragma unroll
+        for (int o = 16; o >= 1; o >>= 1) dot += __shfl_xor_sync(0xffffffffu, dot, o);
+        if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5][0] = dot;
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            float t = 0.f;
+#pragma unroll
+            for (int w = 0; w < NTHR / 32; ++w) t += red[w][0];
+            atomicAdd(dq + d.nc - 1, t);
+        }
+        __syncthreads();
+    }
     for (int c0 = d.nc - 1; c0 >= 0; c0 -= SPB) {   // chunks c0, c0-1, ...
         float4 off[SPB], nxt[SPB];
         float dec[SPB], dot[SPB];
@@ -988,10 +1013,12 @@ __global__ void __launch_bounds__(NTHR) state_pass_bwd_kernel(Dims d, Ws ws, flo
         }
         __syncthreads();
     }
+    if (dinit && ok) reinterpret_cast<float4*>(dinit)[bh4] = run;
 }
 // element-wise fallback (P * N not a multiple of 4)
 template <bool SEQ>
-__global__ void __launch_bounds__(NTHR) state_pass_bwd_kernel_scalar(Dims d, Ws ws, float* dstates, float* dcsQ) {
+__global__ void __launch_bounds__(NTHR) state_pass_bwd_kernel_scalar(Dims d, Ws ws, float* dstates, float* dcsQ, const float* fin,
+                                                                     const float* dfin, float* dinit) {
     __shared__ float red[NTHR / 32];
     const size_t PN = (size_t)d.P * d.N;
     const int nblk = (int)((PN + NTHR - 1) / NTHR);
@@ -999,7 +1026,8 @@ __global__ void __launch_bounds__(NTHR) state_pass_bwd_kernel_scalar(Dims d, Ws 
     const int h = (blockIdx.x / nblk) % d.H, b = blockIdx.x / (nblk * d.H);
     const size_t e = (size_t)blk * NTHR + threadIdx.x;
     const bool ok = e < PN;
-    float run = 0.f;
+    const size_t bh = ((size_t)b * d.H + h) * PN + e;   // this thread's element of a (batch, H, P, N) tensor
+    float run = (dfin && ok) ? dfin[bh] : 0.f;
     for (int c = d.nc - 1; c >= 0; --c) {
         float* s = dstates + (((size_t)b * d.nc + c) * d.H + h) * PN + e;
         float off = 0.f;
@@ -1009,6 +1037,7 @@ __global__ void __launch_bounds__(NTHR) state_pass_bwd_kernel_scalar(Dims d, Ws 
         }
         float dot = 0.f;
         if (ok && c + 1 < d.nc) dot = run * ws.states[(((size_t)b * d.nc + c + 1) * d.H + h) * PN + e];
+        else if (ok && dfin) dot = run * fin[bh];
 #pragma unroll
         for (int o = 16; o >= 1; o >>= 1) dot += __shfl_xor_sync(0xffffffffu, dot, o);
         if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = dot;
@@ -1016,20 +1045,22 @@ __global__ void __launch_bounds__(NTHR) state_pass_bwd_kernel_scalar(Dims d, Ws 
         if (threadIdx.x == 0) {
             float t = 0.f;
             for (int w = 0; w < NTHR / 32; ++w) t += red[w];
-            if (c + 1 < d.nc) atomicAdd(dcsQ + ((size_t)b * d.H + h) * d.nc + c, t);
+            if (c + 1 < d.nc || dfin) atomicAdd(dcsQ + ((size_t)b * d.H + h) * d.nc + c, t);
         }
         __syncthreads();
         const float csQ = ws.cs[(((size_t)b * d.H + h) * d.nc + c) * d.Q + d.Q - 1];
         const float dec = (SEQ && seq_end(d, b, c) != seq_prev(d, b, c)) ? 0.f : exp_acc(csQ);
         run = off + dec * run;
     }
+    if (dinit && ok) dinit[bh] = run;
 }
 
 // ---- B3: Z = (CB o decay)^T dout + exp(cs_Q - cs) B G^T;  dx = dt' Z + D dout;
 //          ddtp_exp[s] = sum_p x Z;  dcs_pos[l] = sum_p dout (out - D x);  dD += sum dout x --------
 template <typename T, bool SEQ>
 __global__ void __launch_bounds__(NTHR, 2) dx_kernel(View4<T> X, View4<T> Bv, View4<T> DO, View4<T> OUT, const float* D, Dims d, Ws ws,
-                                                     const float* G, float* dx, OutS dxs, float* ddtp_exp, float* dcs_pos, float* dD, int x3) {
+                                                     const float* G, float* dx, OutS dxs, float* ddtp_exp, float* dcs_pos, float* dD, int x3,
+                                                     int has_dfin) {
     Smem& sm = smem_ref();
     const int ntm = (d.Q + BM - 1) / BM, ntp = (d.P + BN - 1) / BN;
     int bid = blockIdx.x;
@@ -1066,7 +1097,7 @@ __global__ void __launch_bounds__(NTHR, 2) dx_kernel(View4<T> X, View4<T> Bv, Vi
         __syncthreads();
         warp_mma<true, false>(acc, sm.A[buf], sm.B[buf], x3 != 0);
     }
-    if (c + 1 < d.nc) {  // G of the last chunk is identically zero
+    if (c + 1 < d.nc || has_dfin) {  // G of the last chunk is dfinal_states: zero unless given
         for (int k0 = 0; k0 < d.N; k0 += BK, buf ^= 1) {
             fill_tile<BM, true>(sm.A[buf], b_ifast, [&](int i, int k) {
                 const int s = m0 + i, n = k0 + k;
@@ -1128,7 +1159,8 @@ __global__ void __launch_bounds__(NTHR, 2) dx_kernel(View4<T> X, View4<T> Bv, Vi
 // allows) into UMMA tiles, accumulator row = one thread in the epilogue (row sums need no shuffles).
 template <typename T, bool SEQ>
 __global__ void __launch_bounds__(NTHR, TcEngine::MIN_CTAS) dx_kernel_tc(View4<T> X, View4<T> Bv, View4<T> DO, View4<T> OUT, const float* D, Dims d, Ws ws,
-                                                        const float* G, float* dx, OutS dxs, float* ddtp_exp, float* dcs_pos, float* dD, int x3) {
+                                                        const float* G, float* dx, OutS dxs, float* ddtp_exp, float* dcs_pos, float* dD, int x3,
+                                                        int has_dfin) {
     using E = TcEngine;
     E::Shared& sm = E::smem();
     const int ntm = (d.Q + BM - 1) / BM, ntp = (d.P + BN - 1) / BN;
@@ -1168,7 +1200,7 @@ __global__ void __launch_bounds__(NTHR, TcEngine::MIN_CTAS) dx_kernel_tc(View4<T
             },
             [&](int, const RegTile<BN>& r, const tc::Dst& dst) { E::template store_any<BN>(dst, r, kib, Identity()); });
     }
-    if (c + 1 < d.nc) {   // Z += exp(cs_Q - cs_s) B G^T (G of the last chunk is identically zero)
+    if (c + 1 < d.nc || has_dfin) {   // Z += exp(cs_Q - cs_s) B G^T (G of the last chunk is dfinal_states: zero unless given)
         if (threadIdx.x < BM) {
             const int s = min(m0 + (int)threadIdx.x, d.Q - 1);
             sm.v1[0][threadIdx.x] = exp_acc(csQ - sm.cs[0][s]);
@@ -1272,7 +1304,8 @@ __global__ void __launch_bounds__(NTHR, 2) dcb_kernel(View4<T> X, View4<T> DO, D
 // ---- B5: dC = dCB B + sum_h exp(cs_h) dout_h Sin_h ;  dB = dCB^T C + sum_h exp(cs_Q - cs) dt' x_h G_h ----
 template <typename T, bool SEQ>
 __global__ void __launch_bounds__(NTHR, 2) dbc_kernel(View4<T> X, View4<T> Bv, View4<T> Cv, View4<T> DO, Dims d, Ws ws,
-                                                      const float* dcb_all, const float* G, float* dB, float* dC, OutS dbs, OutS dcs, int x3) {
+                                                      const float* dcb_all, const float* G, float* dB, float* dC, OutS dbs, OutS dcs, int x3,
+                                                      int has_dfin) {
     Smem& sm = smem_ref();
     const int ntm = (d.Q + BM - 1) / BM, ntn = (d.N + BN - 1) / BN;
     int bid = blockIdx.x;
@@ -1323,7 +1356,7 @@ __global__ void __launch_bounds__(NTHR, 2) dbc_kernel(View4<T> X, View4<T> Bv, V
     const View4<T>& Asrc = which == 0 ? DO : X;
     const bool a_ifast = Asrc.s1 <= Asrc.s3;
     const float* Sbase = which == 0 ? ws.states : G;
-    if (which == 0 || c + 1 < d.nc) {
+    if (which == 0 || c + 1 < d.nc || has_dfin) {   // dB: G of the last chunk is dfinal_states, zero unless given
         // dC: only positions of the sequence entering the chunk see Sin; dB: only those of the sequence open at its end feed G
         const int ref = SEQ ? (which == 0 ? seq_prev(d, b, c) : seq_end(d, b, c)) : 0;
         if (SEQ) stage_sid(sm, d, b, c);
@@ -1361,7 +1394,8 @@ __global__ void __launch_bounds__(NTHR, 2) dbc_kernel(View4<T> X, View4<T> Bv, V
 // B5 on the tcgen05 engine.
 template <typename T>
 __global__ void __launch_bounds__(NTHR, TcEngine::MIN_CTAS) dbc_kernel_tc(View4<T> X, View4<T> Bv, View4<T> Cv, View4<T> DO, Dims d, Ws ws,
-                                                         const float* dcb_all, const float* G, float* dB, float* dC, OutS dbs, OutS dcs, int x3) {
+                                                         const float* dcb_all, const float* G, float* dB, float* dC, OutS dbs, OutS dcs, int x3,
+                                                         int has_dfin) {
     using E = TcEngine;
     E::Shared& sm = E::smem();
     const int ntm = (d.Q + BM - 1) / BM, ntn = (d.N + BN - 1) / BN;
@@ -1408,7 +1442,7 @@ __global__ void __launch_bounds__(NTHR, TcEngine::MIN_CTAS) dbc_kernel_tc(View4<
     // state terms, head by head (K = p):  A(i = l, k = p) = src[l][p] w_l,  B(i = n, k = p) = S[p][n]
     const View4<T>& Asrc = which == 0 ? DO : X;
     const float* Sbase = which == 0 ? ws.states : G;
-    if (which == 0 || c + 1 < d.nc) {
+    if (which == 0 || c + 1 < d.nc || has_dfin) {   // dB: G of the last chunk is dfinal_states, zero unless given
         const bool kia = Asrc.s1 == 1;
         for (int hh = 0; hh < d.hpg; ++hh) {
             const int h = g * d.hpg + hh, hb = hh & 1;
@@ -1743,32 +1777,35 @@ static int bwd_masked(const b200_ssd_bwd_params* q, const Dims& d, const Ws& ws,
     else
         LAUNCH((chunk_state_kernel<T, 1, MmaEngine, SEQ>), (size_t)d.batch * d.nc * d.H * ntp64 * ntn128, NTHR, SM, st, DO, Cv, d, ws, sc.dstates,
                x3);
+    const int has_dfin = q->dfinal_states != nullptr;
     {
         const size_t PN = (size_t)d.P * d.N;
         const bool vec = PN % 4 == 0 && ((uintptr_t)ws.states & 15) == 0 && ((uintptr_t)sc.dstates & 15) == 0 &&
-                         (size_t)d.batch * d.H <= 65535;
+                         ((uintptr_t)q->final_states & 15) == 0 && ((uintptr_t)q->dfinal_states & 15) == 0 &&
+                         ((uintptr_t)q->dinitial_states & 15) == 0 && (size_t)d.batch * d.H <= 65535;
         if (vec) {
-            state_pass_bwd_kernel<SEQ><<<dim3((unsigned)((PN / 4 + NTHR - 1) / NTHR), (unsigned)(d.batch * d.H)), NTHR, 0, st>>>(d, ws, sc.dstates,
-                                                                                                                        sc.dcsQ);
+            state_pass_bwd_kernel<SEQ><<<dim3((unsigned)((PN / 4 + NTHR - 1) / NTHR), (unsigned)(d.batch * d.H)), NTHR, 0, st>>>(
+                d, ws, sc.dstates, sc.dcsQ, q->final_states, q->dfinal_states, q->dinitial_states);
             if (int rc_ = check_launch("state_pass_bwd_kernel")) return rc_;
         } else {
             const int nblk = (int)((PN + NTHR - 1) / NTHR);
-            LAUNCH(state_pass_bwd_kernel_scalar<SEQ>, (size_t)d.batch * d.H * nblk, NTHR, 0, st, d, ws, sc.dstates, sc.dcsQ);
+            LAUNCH(state_pass_bwd_kernel_scalar<SEQ>, (size_t)d.batch * d.H * nblk, NTHR, 0, st, d, ws, sc.dstates, sc.dcsQ, q->final_states,
+                   q->dfinal_states, q->dinitial_states);
         }
     }
     if (use_tcgen05())
         LAUNCH((dx_kernel_tc<T, SEQ>), (size_t)d.batch * d.nc * d.H * ntq128 * ntp64, NTHR, (x3 ? tc::SMEM_X3 : tc::SMEM_TF32), st, X, Bv, DO, OUT,
-               p->D, d, ws, sc.dstates, q->dx, dxs, sc.ddtp_exp, sc.dcs_pos, q->dD, x3);
+               p->D, d, ws, sc.dstates, q->dx, dxs, sc.ddtp_exp, sc.dcs_pos, q->dD, x3, has_dfin);
     else
         LAUNCH((dx_kernel<T, SEQ>), (size_t)d.batch * d.nc * d.H * ntq128 * ntp64, NTHR, SM, st, X, Bv, DO, OUT, p->D, d, ws, sc.dstates, q->dx,
-               dxs, sc.ddtp_exp, sc.dcs_pos, q->dD, x3);
+               dxs, sc.ddtp_exp, sc.dcs_pos, q->dD, x3, has_dfin);
     LAUNCH((dcb_kernel<T, SEQ>), (size_t)d.batch * d.nc * d.G * ntq128 * ntq64, NTHR, SM, st, X, DO, d, ws, sc.dcb, x3);
     if (use_tcgen05())
         LAUNCH((dbc_kernel_tc<T>), (size_t)d.batch * d.nc * d.G * ntq128 * ntn64 * 2, NTHR, (x3 ? tc::SMEM_X3 : tc::SMEM_TF32), st, X, Bv, Cv, DO, d,
-               ws, sc.dcb, sc.dstates, q->dB, q->dC, dbs, dcs, x3);
+               ws, sc.dcb, sc.dstates, q->dB, q->dC, dbs, dcs, x3, has_dfin);
     else
         LAUNCH((dbc_kernel<T, SEQ>), (size_t)d.batch * d.nc * d.G * ntq128 * ntn64 * 2, NTHR, SM, st, X, Bv, Cv, DO, d, ws, sc.dcb, sc.dstates,
-               q->dB, q->dC, dbs, dcs, x3);
+               q->dB, q->dC, dbs, dcs, x3, has_dfin);
     return 0;
 }
 
@@ -1849,6 +1886,10 @@ extern "C" int b200_ssd_bwd(const b200_ssd_bwd_params* q, b200_stream_t stream) 
     B200_REQUIRE(q->dout && q->dx && q->ddt && q->dB && q->dC && q->dA && q->scratch,
                  "b200_ssd_bwd: dout/dx/ddt/dB/dC/dA/scratch must be non-NULL");
     B200_REQUIRE((reinterpret_cast<uintptr_t>(q->scratch) & 15) == 0, "b200_ssd_bwd: scratch must be 16-byte aligned");
+    B200_REQUIRE(q->dfinal_states == nullptr || q->final_states != nullptr,
+                 "b200_ssd_bwd: dfinal_states needs the forward's final_states");
+    B200_REQUIRE(q->dinitial_states == nullptr || q->f.initial_states != nullptr,
+                 "b200_ssd_bwd: dinitial_states needs f.initial_states");
     cudaStream_t st = (cudaStream_t)stream;
     switch (q->f.io_dtype) {
         case B200_F32: return bwd_impl<float>(q, st);

@@ -11,9 +11,15 @@ dt_bias (H); initial_states (batch, H, P, N).  Returns out (batch, L, H, P) in x
 whatever strides they have (the reference passes (b, l, .) views of channel-major storage, L stride 1)
 -- nothing is copied.
 
+Gradients flow into initial_states (in its dtype) and out of final_states, as in mamba_ssm 2.2.2, so a
+long sequence can be trained over several calls that pass the state along; varlen_states carries none.
+A backward that needs neither runs exactly the kernels it would without them.
+
 Packed sequences: seq_idx (batch, L) integers, non-decreasing along L (the caller's contract, not
 checked: that would need a host sync), restarts the recurrence wherever it changes, in the forward
-and in the backward; initial_states[b] reach row b's first sequence only when its id is 0.
+and in the backward; initial_states[b] reach row b's first sequence only when its id is 0 (so only
+such a row gets a non-zero initial_states gradient), and the final_states gradient reaches only the
+row's last sequence.
 return_varlen_states (batch 1, cu_seqlens (nseq + 1,) giving the same boundaries) also returns the
 state after each sequence's last token.  It differs from mamba_ssm in one case: a first sequence that
 ends inside the first chunk includes initial_states, as out and final_states do.
@@ -124,24 +130,29 @@ class SsdChunkScanFn(torch.autograd.Function):
             if nseq > 0:
                 _lib.launch("b200_ssd_varlen_states", dev, ctypes.byref(p), cu_seqlens.data_ptr(), nseq, varlen.data_ptr())
             extra += (varlen,)
-        ctx.save_for_backward(x, dt_, A32, B_, C_, D32, bias32, init32, seq_idx, out, ws)
+        ctx.save_for_backward(x, dt_, A32, B_, C_, D32, bias32, init32, seq_idx, out, ws, fin)
         ctx.cfg = (chunk_size, bool(dt_softplus), tuple(dt_limit), prec)
         ctx.dtypes = (dt.dtype, A.dtype, B.dtype, C.dtype, None if D is None else D.dtype,
-                      None if dt_bias is None else dt_bias.dtype)
-        if extra:
-            ctx.mark_non_differentiable(*extra)
-            return (out,) + extra
-        return out
+                      None if dt_bias is None else dt_bias.dtype, None if initial_states is None else initial_states.dtype)
+        # an output the loss does not use arrives in backward as None (not a zero tensor), so a final_states that takes
+        # no part in the loss costs nothing
+        ctx.set_materialize_grads(False)
+        if cu_seqlens is not None:
+            ctx.mark_non_differentiable(extra[-1])
+        return (out,) + extra if extra else out
 
     @staticmethod
     @_no_autocast
-    def backward(ctx, dout, *unused):
-        x, dt_, A32, B_, C_, D32, bias32, init32, seq_idx, out, ws = ctx.saved_tensors
+    def backward(ctx, dout, *dextra):
+        x, dt_, A32, B_, C_, D32, bias32, init32, seq_idx, out, ws, fin = ctx.saved_tensors
+        dfin = dextra[0] if fin is not None else None
         chunk_size, dt_softplus, dt_limit, precision = ctx.cfg
         batch, L, H, P = x.shape
         G, N = B_.shape[2], B_.shape[3]
         dev = x.device
-        dout = dout.to(x.dtype)
+        dout = torch.zeros_like(out) if dout is None else dout.to(x.dtype)
+        dfin = None if dfin is None else _lib.f32c(dfin)
+        dinit = torch.empty_like(init32) if ctx.needs_input_grad[7] else None
         # every gradient in the layout of its primal (the models pass sequence-contiguous views of channel-major storage,
         # SSD/MedSSD.py:344-347): the cross-scan adjoint then reads them in place -- no strided copy after the kernels
         dx, ddt, dB, dC = (_empty_like_layout(t) for t in (x, dt_, B_, C_))
@@ -159,16 +170,17 @@ class SsdChunkScanFn(torch.autograd.Function):
         q.dx_stride[:], q.ddt_stride[:] = list(dx.stride()), list(ddt.stride())
         q.dB_stride[:], q.dC_stride[:] = list(dB.stride()), list(dC.stride())
         q.dA, q.dD, q.ddt_bias, q.scratch = dA.data_ptr(), _lib.ptr(dD), _lib.ptr(dbias), scratch.data_ptr()
+        q.final_states, q.dfinal_states, q.dinitial_states = _lib.ptr(fin), _lib.ptr(dfin), _lib.ptr(dinit)
         prof = _profiler
         with torch.cuda.device(dev):
             tok = prof.begin() if prof is not None else None
             _lib.launch("b200_ssd_bwd", dev, ctypes.byref(q))
             if prof is not None:
                 prof.end(tok, "bwd", (batch, L, H, P, G, N, chunk_size, precision))
-        t_dt, t_A, t_B, t_C, t_D, t_bias = ctx.dtypes
+        t_dt, t_A, t_B, t_C, t_D, t_bias, t_init = ctx.dtypes
         return (dx.to(x.dtype), ddt.to(t_dt), dA.to(t_A), dB.to(t_B), dC.to(t_C),
                 None if dD is None else dD.to(t_D), None if dbias is None else dbias.to(t_bias),
-                None, None, None, None, None, None, None, None)
+                None if dinit is None else dinit.to(t_init), None, None, None, None, None, None, None)
 
 
 def mamba_chunk_scan_combined(x, dt, A, B, C, chunk_size, D=None, z=None, dt_bias=None, initial_states=None,
@@ -185,7 +197,8 @@ def mamba_chunk_scan_combined(x, dt, A, B, C, chunk_size, D=None, z=None, dt_bia
     Return:
         out: (batch, seqlen, nheads, headdim) [, final_states (batch, nheads, headdim, dstate)]
         [, varlen_states (nseq, nheads, headdim, dstate): the state after each sequence's last token]
-    final_states and varlen_states are fp32 and carry no gradient.
+    final_states and varlen_states are fp32.  initial_states receives a gradient in its own dtype, and final_states
+    passes one back (with seq_idx: to row b's leading id-0 sequence and from its last sequence); varlen_states carries none.
     """
     _lib.require_cuda(x, dt, A, B, C, D, z, dt_bias, initial_states, seq_idx)
     if x.dim() != 4 or dt.dim() != 3 or B.dim() != 4 or C.dim() != 4:
@@ -202,8 +215,6 @@ def mamba_chunk_scan_combined(x, dt, A, B, C, chunk_size, D=None, z=None, dt_bia
     if initial_states is not None:
         if tuple(initial_states.shape) != (batch, H, P, N):
             raise RuntimeError(f"mamba_chunk_scan_combined: initial_states must be {(batch, H, P, N)}")
-        if initial_states.requires_grad:
-            raise NotImplementedError("mamba_chunk_scan_combined: no gradient for initial_states in the B200 kernels")
     seq_idx = _index_tensor(seq_idx, "seq_idx", x.device, (batch, L))
     if return_varlen_states:
         if cu_seqlens is None:
