@@ -379,6 +379,32 @@ int b200_shuffle_cat_add_bwd(const void* dout, int32_t io_dtype, void* dleft, in
 int b200_patch_merge(const void* x, void* out, int32_t batch, int32_t H, int32_t W, int32_t pixel_bytes, int32_t inverse,
                      b200_stream_t stream);
 
+/* ------------------------------------------------------------------------------------------
+ * Causal depth-wise conv1d (+ bias, + SiLU): causal-conv1d's causal_conv1d_fn, the conv of mamba_ssm 2.2.2's
+ * mamba_split_conv1d_scan_combined.  Channel c of x (batch, seqlen, dim), width in 2..4, fp32 arithmetic:
+ *   out[b, t, c] = act(bias[c] + sum_k weight[c, k] * x[b, t - (width-1) + k, c]),   act = silu if silu != 0, else identity,
+ * with x before t = 0 taken as zero and, when seq_idx (batch, seqlen) int32 is given, a tap skipped unless its seq_idx equals t's.
+ *   x (x_dtype in {F32, BF16, F16}) and out (out_dtype) are channel-last views with channel stride 1 and the given batch / time
+ *   strides, read and written in place (x may be a column slice of in_proj's output with any pitch); weight (dim, width) and bias
+ *   (dim) f32 contiguous, bias may be NULL.
+ * Backward: dout (batch, seqlen, dim) f32, the gradient of out (after the activation), with its own batch / time strides ->
+ *   dx in x_dtype through its strides, dweight_partial (P, dim, width) and dbias_partial (P, dim) f32 per-CTA partial sums with
+ *   P = b200_causal_conv1d_partials(batch, seqlen, dim, width), which the caller adds up over P (no atomics: reproducible);
+ *   dbias_partial may be NULL.  The pre-activation is recomputed from x, weight and bias.
+ * Bad sizes, width, dtype codes, NULL required pointers or negative strides return < 0 with a message and launch nothing
+ * (b200_causal_conv1d_partials too).
+ * ------------------------------------------------------------------------------------------ */
+int b200_causal_conv1d_partials(int32_t batch, int32_t seqlen, int32_t dim, int32_t width);
+int b200_causal_conv1d_fwd(const void* x, int32_t x_dtype, int64_t x_batch_stride, int64_t x_seq_stride, const float* weight,
+                           const float* bias, const int32_t* seq_idx, int64_t seq_batch_stride, int64_t seq_stride, void* out,
+                           int32_t out_dtype, int64_t out_batch_stride, int64_t out_seq_stride, int32_t batch, int32_t seqlen,
+                           int32_t dim, int32_t width, int32_t silu, b200_stream_t stream);
+int b200_causal_conv1d_bwd(const float* dout, int64_t dout_batch_stride, int64_t dout_seq_stride, const void* x, int32_t x_dtype,
+                           int64_t x_batch_stride, int64_t x_seq_stride, const float* weight, const float* bias,
+                           const int32_t* seq_idx, int64_t seq_batch_stride, int64_t seq_stride, void* dx, int64_t dx_batch_stride,
+                           int64_t dx_seq_stride, float* dweight_partial, float* dbias_partial, int32_t batch, int32_t seqlen,
+                           int32_t dim, int32_t width, int32_t silu, b200_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------ */
 const char* b200_last_error(void);   /* thread-local message of the last failing call */
 int b200_version(void);              /* ABI version, bumped on any struct change */

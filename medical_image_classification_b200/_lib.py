@@ -113,6 +113,10 @@ SIGNATURES = {
     "b200_shuffle_cat_add_fwd": (C.c_int, [vp, i32, vp, i32, vp, vp, i32, i32, i32, i32, vp]),
     "b200_shuffle_cat_add_bwd": (C.c_int, [vp, i32, vp, i32, vp, i32, i32, i32, i32, vp]),
     "b200_patch_merge": (C.c_int, [vp, vp, i32, i32, i32, i32, i32, vp]),
+    "b200_causal_conv1d_partials": (C.c_int, [i32] * 4),
+    "b200_causal_conv1d_fwd": (C.c_int, [vp, i32, i64, i64, vp, vp, vp, i64, i64, vp, i32, i64, i64, i32, i32, i32, i32, i32, vp]),
+    "b200_causal_conv1d_bwd": (C.c_int, [vp, i64, i64, vp, i32, i64, i64, vp, vp, vp, i64, i64, vp, i64, i64, vp, vp, i32, i32, i32,
+                                         i32, i32, vp]),
     "b200_last_error": (C.c_char_p, []),
     "b200_version": (C.c_int, []),
     "b200_kernel_launches": (C.c_int, []),

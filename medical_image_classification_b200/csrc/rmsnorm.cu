@@ -32,65 +32,6 @@ constexpr int RN_CTAS = 148 * 8;         // 2048 threads per SM
 
 __device__ __forceinline__ float rn_silu(float z) { return z / (1.f + expf(-z)); }
 
-// V consecutive elements as raw bits: the loads of a row are all issued before the first conversion (rn_cvt)
-template <int V>
-__device__ __forceinline__ void rn_ld(const void* base, int64_t idx, int dt, uint32_t (&r)[V]) {
-    if (dt == B200_F32) {
-        const float* p = static_cast<const float*>(base) + idx;
-        if constexpr (V == 4) {
-            const uint4 u = __ldcs(reinterpret_cast<const uint4*>(p));
-            r[0] = u.x, r[1] = u.y, r[2] = u.z, r[3] = u.w;
-        } else if constexpr (V == 2) {
-            const uint2 u = __ldcs(reinterpret_cast<const uint2*>(p));
-            r[0] = u.x, r[1] = u.y;
-        } else {
-            r[0] = __ldcs(reinterpret_cast<const unsigned int*>(p));
-        }
-    } else {
-        const unsigned short* p = static_cast<const unsigned short*>(base) + idx;
-        if constexpr (V == 4) {
-            const uint2 u = __ldcs(reinterpret_cast<const uint2*>(p));
-            r[0] = u.x, r[1] = u.y;
-        } else if constexpr (V == 2) {
-            r[0] = __ldcs(reinterpret_cast<const unsigned int*>(p));
-        } else {
-            r[0] = __ldcs(p);
-        }
-    }
-}
-
-template <int V>
-__device__ __forceinline__ void rn_cvt(const uint32_t (&r)[V], int dt, float* v) {
-#pragma unroll
-    for (int j = 0; j < V; ++j) {
-        if (dt == B200_F32) {
-            v[j] = __uint_as_float(r[j]);
-        } else {
-            const uint32_t h = V == 1 ? r[0] & 0xffffu : (r[j >> 1] >> (16 * (j & 1))) & 0xffffu;
-            v[j] = dt == B200_BF16 ? __uint_as_float(h << 16) : __half2float(__ushort_as_half((unsigned short)h));
-        }
-    }
-}
-
-template <int V>
-__device__ __forceinline__ void rn_st(void* base, int64_t idx, int dt, const float* v) {
-    if (dt == B200_F32) {
-        float* p = static_cast<float*>(base) + idx;
-        if constexpr (V == 4) __stcs(reinterpret_cast<float4*>(p), make_float4(v[0], v[1], v[2], v[3]));
-        else if constexpr (V == 2) __stcs(reinterpret_cast<float2*>(p), make_float2(v[0], v[1]));
-        else __stcs(p, v[0]);
-        return;
-    }
-    uint32_t h[V];
-#pragma unroll
-    for (int j = 0; j < V; ++j)
-        h[j] = dt == B200_BF16 ? __bfloat16_as_ushort(__float2bfloat16_rn(v[j])) : __half_as_ushort(__float2half_rn(v[j]));
-    unsigned short* p = static_cast<unsigned short*>(base) + idx;
-    if constexpr (V == 4) __stcs(reinterpret_cast<uint2*>(p), make_uint2(h[0] | h[1] << 16, h[2] | h[3] << 16));
-    else if constexpr (V == 2) __stcs(reinterpret_cast<unsigned int*>(p), h[0] | h[1] << 16);
-    else __stcs(p, (unsigned short)h[0]);
-}
-
 // sum over a team: a warp, or the whole CTA (then every thread of the CTA calls it at the same point)
 template <int T>
 __device__ __forceinline__ float rn_team_sum(float v, float* sbuf) {
