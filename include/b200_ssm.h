@@ -405,11 +405,64 @@ int b200_causal_conv1d_bwd(const float* dout, int64_t dout_batch_stride, int64_t
                            int64_t dx_seq_stride, float* dweight_partial, float* dbias_partial, int32_t batch, int32_t seqlen,
                            int32_t dim, int32_t width, int32_t silu, b200_stream_t stream);
 
+/* One decoding step of the same conv: causal-conv1d's causal_conv1d_update without cache_seqlens.  x (batch, dim, seqlen) is the
+ * next seqlen inputs, conv_state (batch, dim, state_len) the last state_len inputs before them (state_len >= width - 1), both in
+ * x_dtype and read through their strides (x may be a column slice of in_proj's output).  Over v = cat(conv_state, x) along time:
+ *   out[b, c, t] = act(bias[c] + sum_k weight[c, k] * v[b, c, state_len + t - (width-1) + k]),   t < seqlen,
+ * and conv_state is overwritten in place with the last state_len columns of v (also when seqlen > state_len).  out (batch, dim,
+ * seqlen) in x_dtype through its strides; weight (dim, width) and bias (dim) in their own dtypes through their strides, bias may
+ * be NULL.  Same error rules as above. */
+int b200_causal_conv1d_update(const void* x, int32_t x_dtype, int64_t x_batch_stride, int64_t x_dim_stride, int64_t x_seq_stride,
+                              void* conv_state, int64_t state_batch_stride, int64_t state_dim_stride, int64_t state_seq_stride,
+                              const void* weight, int32_t weight_dtype, int64_t weight_dim_stride, int64_t weight_width_stride,
+                              const void* bias, int32_t bias_dtype, int64_t bias_stride, void* out, int64_t out_batch_stride,
+                              int64_t out_dim_stride, int64_t out_seq_stride, int32_t batch, int32_t dim, int32_t seqlen,
+                              int32_t state_len, int32_t width, int32_t silu, b200_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------
+ * One recurrent step of a Mamba state: mamba_ssm 2.2.2's selective_state_update (the decode step of Mamba2.step and of
+ * transformers' Mamba2Mixer).  For batch b, head h, row p < headdim, n < dstate, group g = h / (nheads / ngroups), fp32:
+ *   dt'  = softplus?(dt[b,h,p] + dt_bias[h,p])                     (x <= 20 ? log1p(exp x) : x)
+ *   state[b,h,p,n] <- state[b,h,p,n] * exp(A[h,p,n] dt') + B[b,g,n] dt' x[b,h,p]          (in place, in state_dtype)
+ *   out[b,h,p] = (sum_n state[b,h,p,n] C[b,g,n] + D[h,p] x[b,h,p]) * silu(z[b,h,p])
+ * with the fp32 updated state in the sum; D, z, dt_bias are optional (NULL).  Mamba-1's form is nheads = 1.  Every tensor is
+ * read (state and out written) in place through its element strides, which may be 0 (an expanded A, dt, dt_bias or D), in its
+ * own dtype.  When A, dt and dt_bias are constant over (p, n), exp(A dt') is formed once per (batch, head).  dstate <= 256.
+ * Bad sizes, dtype codes, NULL required pointers or negative strides return < 0 with a message and launch nothing.
+ * ------------------------------------------------------------------------------------------ */
+typedef struct {
+    int32_t batch, nheads, headdim, ngroups, dstate;
+    int32_t dt_softplus;
+    int32_t state_dtype, x_dtype, dt_dtype, A_dtype, B_dtype, C_dtype, D_dtype, z_dtype, dt_bias_dtype, out_dtype;
+    int64_t state_stride[4];   /* batch, head, p, n */
+    int64_t x_stride[3];       /* batch, head, p */
+    int64_t dt_stride[3];      /* batch, head, p */
+    int64_t A_stride[3];       /* head, p, n */
+    int64_t B_stride[3];       /* batch, group, n */
+    int64_t C_stride[3];       /* batch, group, n */
+    int64_t D_stride[2];       /* head, p */
+    int64_t z_stride[3];       /* batch, head, p */
+    int64_t dt_bias_stride[2]; /* head, p */
+    int64_t out_stride[3];     /* batch, head, p */
+    void* state;
+    const void* x;
+    const void* dt;
+    const void* A;
+    const void* B;
+    const void* C;
+    const void* D;       /* or NULL */
+    const void* z;       /* or NULL */
+    const void* dt_bias; /* or NULL */
+    void* out;
+} b200_ssu_params;
+
+int b200_selective_state_update(const b200_ssu_params* p, b200_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------ */
 const char* b200_last_error(void);   /* thread-local message of the last failing call */
 int b200_version(void);              /* ABI version, bumped on any struct change */
 int b200_kernel_launches(void);      /* number of kernels this library has launched in this process */
-size_t b200_sizeof_params(int32_t which); /* 0 sscan_fwd, 1 sscan_bwd, 2 ssd_fwd, 3 ssd_bwd: lets a binding check its struct layout */
+size_t b200_sizeof_params(int32_t which); /* 0 sscan_fwd, 1 sscan_bwd, 2 ssd_fwd, 3 ssd_bwd, 4 ssu: lets a binding check its struct layout */
 
 #ifdef __cplusplus
 }

@@ -74,6 +74,18 @@ class SsdBwdParams(C.Structure):
     ]
 
 
+class SsuParams(C.Structure):
+    """b200_ssu_params."""
+    _fields_ = [
+        ("batch", i32), ("nheads", i32), ("headdim", i32), ("ngroups", i32), ("dstate", i32), ("dt_softplus", i32),
+        ("state_dtype", i32), ("x_dtype", i32), ("dt_dtype", i32), ("A_dtype", i32), ("B_dtype", i32), ("C_dtype", i32),
+        ("D_dtype", i32), ("z_dtype", i32), ("dt_bias_dtype", i32), ("out_dtype", i32),
+        ("state_stride", i64 * 4), ("x_stride", i64 * 3), ("dt_stride", i64 * 3), ("A_stride", i64 * 3), ("B_stride", i64 * 3),
+        ("C_stride", i64 * 3), ("D_stride", i64 * 2), ("z_stride", i64 * 3), ("dt_bias_stride", i64 * 2), ("out_stride", i64 * 3),
+        ("state", vp), ("x", vp), ("dt", vp), ("A", vp), ("B", vp), ("C", vp), ("D", vp), ("z", vp), ("dt_bias", vp), ("out", vp),
+    ]
+
+
 _DTYPES = {torch.float32: 0, torch.bfloat16: 1, torch.float16: 2}
 
 # name -> (restype, argtypes) of every function include/b200_ssm.h declares, in the header's order
@@ -117,6 +129,10 @@ SIGNATURES = {
     "b200_causal_conv1d_fwd": (C.c_int, [vp, i32, i64, i64, vp, vp, vp, i64, i64, vp, i32, i64, i64, i32, i32, i32, i32, i32, vp]),
     "b200_causal_conv1d_bwd": (C.c_int, [vp, i64, i64, vp, i32, i64, i64, vp, vp, vp, i64, i64, vp, i64, i64, vp, vp, i32, i32, i32,
                                          i32, i32, vp]),
+    "b200_causal_conv1d_update": (C.c_int, [vp, i32, i64, i64, i64, vp, i64, i64, i64, vp, i32, i64, i64, vp, i32, i64, vp, i64, i64,
+                                            i64, i32, i32, i32, i32, i32, i32, vp]),
+    # tests/test_abi.py maps a struct pointer it does not know to c_void_p; the call passes ctypes.byref(SsuParams)
+    "b200_selective_state_update": (C.c_int, [vp, vp]),
     "b200_last_error": (C.c_char_p, []),
     "b200_version": (C.c_int, []),
     "b200_kernel_launches": (C.c_int, []),
@@ -148,7 +164,7 @@ def load() -> C.CDLL:
     for name, (restype, argtypes) in SIGNATURES.items():
         fn = getattr(lib, name)
         fn.restype, fn.argtypes = restype, argtypes
-    for which, st in enumerate((SScanFwdParams, SScanBwdParams, SsdFwdParams, SsdBwdParams)):
+    for which, st in enumerate((SScanFwdParams, SScanBwdParams, SsdFwdParams, SsdBwdParams, SsuParams)):
         if lib.b200_sizeof_params(which) != C.sizeof(st):
             raise RuntimeError(f"libb200ssm ABI mismatch for {st.__name__}: "
                                f"C {lib.b200_sizeof_params(which)} vs ctypes {C.sizeof(st)}")

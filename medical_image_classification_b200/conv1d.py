@@ -9,7 +9,11 @@ out[:, c, t] = act(bias[c] + sum_k weight[c, k] x[:, c, t - (width-1) + k]), act
 (x.stride(1) == 1, e.g. a transposed slice of in_proj's output); otherwise one channel-last copy is made.  Differentiable in x,
 weight and bias.  The conv states (initial_states, return_final_states, final_states_out) are not implemented.
 
-The work is done by csrc/conv1d.cu through b200_causal_conv1d_fwd / _bwd; there is no CPU path.
+    causal_conv1d_update(x, conv_state, weight, bias=None, activation=None, cache_seqlens=None)
+
+is causal-conv1d's decoding step: the conv over cat(conv_state, x) for the new tokens, with conv_state shifted in place.
+
+The work is done by csrc/conv1d.cu through b200_causal_conv1d_fwd / _bwd / _update; there is no CPU path.
 """
 from __future__ import annotations
 
@@ -115,3 +119,38 @@ def causal_conv1d_fn(x, weight, bias=None, seq_idx=None, initial_states=None, re
     if xt.stride(2) != 1:
         xt = xt.contiguous()
     return CausalConv1dFn.apply(xt, weight, bias, seq_idx, silu).transpose(1, 2)
+
+
+@torch.no_grad()
+def causal_conv1d_update(x, conv_state, weight, bias=None, activation=None, cache_seqlens=None):
+    """causal-conv1d's causal_conv1d_update (one decoding step): x (batch, dim) or (batch, dim, seqlen), conv_state (batch, dim,
+    state_len) with state_len >= width - 1, in x's dtype.  Over cat(conv_state, x) along time, returns the conv (+ SiLU for
+    "silu" / "swish") of the last seqlen steps, shaped and typed like x, and overwrites conv_state in place with the last
+    state_len columns.  Every tensor is read through its strides in its own dtype; one kernel launch, not differentiable.
+    cache_seqlens (the circular-buffer mode) is not implemented."""
+    if cache_seqlens is not None:
+        raise NotImplementedError("causal_conv1d_update: cache_seqlens (the circular-buffer conv state) is not implemented")
+    silu = act_is_silu(activation)
+    _lib.require_cuda(x, conv_state, weight, bias)
+    if x.dim() not in (2, 3):
+        raise RuntimeError(f"causal_conv1d_update: x must be (batch, dim) or (batch, dim, seqlen), got {tuple(x.shape)}")
+    x3 = x.unsqueeze(-1) if x.dim() == 2 else x
+    batch, dim, seqlen = x3.shape
+    check_weight(weight, bias, dim, "causal_conv1d_update")
+    width = weight.shape[1]
+    if conv_state.dim() != 3 or tuple(conv_state.shape[:2]) != (batch, dim):
+        raise RuntimeError(f"causal_conv1d_update: conv_state must be ({batch}, {dim}, state_len), got {tuple(conv_state.shape)}")
+    state_len = conv_state.shape[2]
+    if state_len < width - 1:
+        raise RuntimeError(f"causal_conv1d_update: conv_state has state_len {state_len} < width - 1 = {width - 1}")
+    if conv_state.dtype != x.dtype:
+        raise RuntimeError(f"causal_conv1d_update: conv_state dtype {conv_state.dtype} differs from x's {x.dtype}")
+    if any(st == 0 and sz > 1 for sz, st in zip(conv_state.shape, conv_state.stride())):
+        raise RuntimeError("causal_conv1d_update: conv_state has a stride-0 (expanded) dimension and cannot be updated in place")
+    out = torch.empty(x3.shape, dtype=x.dtype, device=x.device)
+    code = _lib.dtype_code(x.dtype)
+    _lib.launch("b200_causal_conv1d_update", x.device, x3.data_ptr(), code, *x3.stride(), conv_state.data_ptr(), *conv_state.stride(),
+                weight.data_ptr(), _lib.dtype_code(weight.dtype), *weight.stride(), _lib.ptr(bias),
+                0 if bias is None else _lib.dtype_code(bias.dtype), 0 if bias is None else bias.stride(0), out.data_ptr(), *out.stride(),
+                batch, dim, seqlen, state_len, width, int(silu))
+    return out if x.dim() == 3 else out.squeeze(-1)

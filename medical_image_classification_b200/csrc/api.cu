@@ -53,7 +53,7 @@ cudaError_t func_attr_per_device(const void* kernel, cudaFuncAttribute attr, int
 }  // namespace b200
 
 extern "C" const char* b200_last_error(void) { return b200::g_err; }
-extern "C" int b200_version(void) { return 3; }
+extern "C" int b200_version(void) { return 4; }
 extern "C" int b200_kernel_launches(void) { return b200::g_launches.load(std::memory_order_relaxed); }
 extern "C" size_t b200_sizeof_params(int32_t which) {
     switch (which) {
@@ -61,6 +61,7 @@ extern "C" size_t b200_sizeof_params(int32_t which) {
         case 1: return sizeof(b200_sscan_bwd_params);
         case 2: return sizeof(b200_ssd_fwd_params);
         case 3: return sizeof(b200_ssd_bwd_params);
+        case 4: return sizeof(b200_ssu_params);
         default: return 0;
     }
 }

@@ -237,6 +237,58 @@ __global__ void __launch_bounds__(CV_THREADS) causal_conv1d_bwd_kernel(const Con
     }
 }
 
+// One decoding step (causal_conv1d_update): a thread per (channel, batch row) walks the seqlen new inputs with the last W-1 values
+// of v = cat(conv_state, x) in registers, then shifts conv_state left by seqlen in place.  The shift reads column j + seqlen before
+// it writes column j, and every column it reads at or after j + seqlen is still unwritten, so one thread needs no staging.
+struct ConvUpdateArgs {
+    const void* x;
+    void* st;
+    const void* w;
+    const void* b;
+    void* y;
+    int64_t xb, xc, xl, sb, sc, sl, wc, wk, bs, yb, yc, yl;
+    int C, L, S, dt, w_dt, b_dt, silu;
+};
+
+__device__ __forceinline__ float cv_ld1(const void* base, int64_t idx, int dt) {
+    uint32_t r[1];
+    float v[1];
+    rn_ld<1>(base, idx, dt, r);
+    rn_cvt<1>(r, dt, v);
+    return v[0];
+}
+
+template <int W>
+__global__ void __launch_bounds__(CV_THREADS) causal_conv1d_update_kernel(const ConvUpdateArgs a) {
+    const int c = blockIdx.x * CV_THREADS + threadIdx.x;
+    if (c >= a.C) return;
+    const int64_t b = blockIdx.y;
+    const int64_t xo = b * a.xb + c * a.xc, so = b * a.sb + c * a.sc, yo = b * a.yb + c * a.yc;
+    float w[W], h[W];
+#pragma unroll
+    for (int k = 0; k < W; ++k) w[k] = cv_ld1(a.w, c * a.wc + k * a.wk, a.w_dt);
+    const float bias = a.b ? cv_ld1(a.b, c * a.bs, a.b_dt) : 0.f;
+#pragma unroll
+    for (int k = 0; k < W - 1; ++k) h[k] = cv_ld1(a.st, so + (a.S - (W - 1) + k) * a.sl, a.dt);
+    for (int t = 0; t < a.L; ++t) {
+        h[W - 1] = cv_ld1(a.x, xo + t * a.xl, a.dt);
+        float acc = bias;
+#pragma unroll
+        for (int k = 0; k < W; ++k) acc = fmaf(w[k], h[k], acc);
+        const float o[1] = {cv_act(acc, a.silu)};
+        rn_st<1>(a.y, yo + t * a.yl, a.dt, o);
+#pragma unroll
+        for (int k = 0; k < W - 1; ++k) h[k] = h[k + 1];
+    }
+    // conv_state <- the last S columns of cat(conv_state, x): column j takes v[j + L] (a 16-bit value survives the fp32 round trip)
+#pragma unroll 1   // unrolled, this loop makes ptxas spill
+    for (int j = 0; j < a.S; ++j) {
+        const int src = j + a.L;
+        const float v[1] = {src < a.S ? cv_ld1(a.st, so + src * a.sl, a.dt) : cv_ld1(a.x, xo + (int64_t)(src - a.S) * a.xl, a.dt)};
+        rn_st<1>(a.st, so + j * a.sl, a.dt, v);
+    }
+}
+
 // ---- host side ----------------------------------------------------------------------------------
 static int cv_esize(int dt) { return dt == B200_F32 ? 4 : 2; }
 static bool cv_dtype_ok(int dt) { return dt == B200_F32 || dt == B200_BF16 || dt == B200_F16; }
@@ -343,4 +395,37 @@ extern "C" int b200_causal_conv1d_bwd(const float* dout, int64_t dout_batch_stri
     const int dts[3] = {x_dtype, B200_F32, x_dtype};
     const int V = cv_vec(dim, 3, ptrs, strides, dts);
     return cv_dispatch<false>(a, width, V, cv_grid(batch, seqlen, dim, V), (cudaStream_t)stream);
+}
+
+extern "C" int b200_causal_conv1d_update(const void* x, int32_t x_dtype, int64_t x_batch_stride, int64_t x_dim_stride, int64_t x_seq_stride,
+                                         void* conv_state, int64_t state_batch_stride, int64_t state_dim_stride, int64_t state_seq_stride,
+                                         const void* weight, int32_t weight_dtype, int64_t weight_dim_stride, int64_t weight_width_stride,
+                                         const void* bias, int32_t bias_dtype, int64_t bias_stride, void* out, int64_t out_batch_stride,
+                                         int64_t out_dim_stride, int64_t out_seq_stride, int32_t batch, int32_t dim, int32_t seqlen,
+                                         int32_t state_len, int32_t width, int32_t silu, b200_stream_t stream) {
+    B200_REQUIRE(x && conv_state && weight && out,
+                 "b200_causal_conv1d_update: NULL argument (x, conv_state, weight and out are required)");
+    B200_REQUIRE(batch >= 1 && batch <= 65535, "b200_causal_conv1d_update: batch = %d outside [1, 65535]", batch);
+    B200_REQUIRE(seqlen >= 1, "b200_causal_conv1d_update: seqlen = %d is not positive", seqlen);
+    B200_REQUIRE(dim >= 1, "b200_causal_conv1d_update: dim = %d is not positive", dim);
+    B200_REQUIRE(width >= 2 && width <= 4, "b200_causal_conv1d_update: width = %d outside [2, 4]", width);
+    B200_REQUIRE(state_len >= width - 1, "b200_causal_conv1d_update: state_len = %d is shorter than width - 1 = %d", state_len, width - 1);
+    B200_REQUIRE(cv_dtype_ok(x_dtype) && cv_dtype_ok(weight_dtype) && (!bias || cv_dtype_ok(bias_dtype)),
+                 "b200_causal_conv1d_update: unsupported dtype x=%d weight=%d bias=%d", x_dtype, weight_dtype, bias_dtype);
+    B200_REQUIRE(x_batch_stride >= 0 && x_dim_stride >= 0 && x_seq_stride >= 0 && state_batch_stride >= 0 && state_dim_stride >= 0 &&
+                     state_seq_stride >= 0 && weight_dim_stride >= 0 && weight_width_stride >= 0 && bias_stride >= 0 &&
+                     out_batch_stride >= 0 && out_dim_stride >= 0 && out_seq_stride >= 0,
+                 "b200_causal_conv1d_update: negative stride");
+    ConvUpdateArgs a{};
+    a.x = x, a.st = conv_state, a.w = weight, a.b = bias, a.y = out;
+    a.xb = x_batch_stride, a.xc = x_dim_stride, a.xl = x_seq_stride, a.sb = state_batch_stride, a.sc = state_dim_stride;
+    a.sl = state_seq_stride, a.wc = weight_dim_stride, a.wk = weight_width_stride, a.bs = bias_stride;
+    a.yb = out_batch_stride, a.yc = out_dim_stride, a.yl = out_seq_stride;
+    a.C = dim, a.L = seqlen, a.S = state_len, a.dt = x_dtype, a.w_dt = weight_dtype, a.b_dt = bias_dtype, a.silu = silu != 0;
+    const dim3 grid((unsigned)((dim + CV_THREADS - 1) / CV_THREADS), (unsigned)batch);
+    const cudaStream_t st = (cudaStream_t)stream;
+    if (width == 2) causal_conv1d_update_kernel<2><<<grid, CV_THREADS, 0, st>>>(a);
+    else if (width == 3) causal_conv1d_update_kernel<3><<<grid, CV_THREADS, 0, st>>>(a);
+    else causal_conv1d_update_kernel<4><<<grid, CV_THREADS, 0, st>>>(a);
+    return check_launch("causal_conv1d_update_kernel");
 }
